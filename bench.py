@@ -8,6 +8,7 @@ node per GPU, 1 local epoch per round on synthetic ImageNet-shape data, random-i
     python bench.py --impl stock_graph ...                   # stock layers / torch.optim / NCCL, local step in ONE CUDA graph
     python bench.py --impl reference ...                     # the unmodified reference (unavailable, see DESIGN.md)
     python bench.py --model bert_base|llama3_8b_lora|glm ...
+    python bench.py --dump-outputs DIR ...                   # also write the last timed step's outputs as DIR/<name>.npy
 
 A bench "step" is ONE federated round = `local_steps` local optimizer steps on every node + the server aggregation
 (weighted FedAvg reduce + server optimizer + broadcast of the new global); for the GLM one step is one federated
@@ -57,7 +58,28 @@ def parse(argv=None):
                     help="fused: K1 -- the first-consumer weights arrive inside the first forward GEMM of the round (transformers, >= 2 GPUs)")
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--no-graph", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the measured arm computed in its last step (the round's loss and "
+                         "the new global model; for the GLM the loss and coefficients) as float32 DIR/<name>.npy")
     return ap.parse_args(argv)
+
+
+DUMP_MAX_ELEMS = 1 << 23        # 32 MB of float32: a larger output is written as a fixed, seeded sample of its elements
+
+
+def dump_outputs(out_dir, arrays):
+    """Write each tensor of ``arrays`` as float32 ``out_dir/<name>.npy``.  The sample of an output larger than
+    DUMP_MAX_ELEMS takes the same (sorted) flat indices on every run, so two builds can be compared element for element."""
+    import numpy as np
+    import torch
+
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in arrays.items():
+        t = t.detach()
+        if t.numel() > DUMP_MAX_ELEMS:
+            idx = torch.randperm(t.numel(), generator=torch.Generator().manual_seed(0))[:DUMP_MAX_ELEMS].sort().values
+            t = t.reshape(-1)[idx.to(t.device)]
+        np.save(os.path.join(out_dir, f"{name}.npy"), t.float().cpu().numpy())
 
 
 def reference_unavailable():
@@ -161,6 +183,8 @@ def run_trainer_arm(impl, args, rank, world, local_rank, device):
         ms = timer.stop()
         barrier_sync(device)
     ms = max_over_ranks(ms, device)
+    if args.dump_outputs and impl == args.impl and rank == 0:       # before the aggregation-only and e2e passes move the model
+        dump_outputs(args.dump_outputs, {"loss": loss, "global_model": trainer.fm.flat[: trainer.fm.n_total]})
     loss_val = float(loss.item())
     if os.environ.get("V6_PROFILE_RANGE") and impl == "b200":      # ncu --profile-from-start off: one more round
         torch.cuda.synchronize()
@@ -226,9 +250,9 @@ def run_glm_arm(impl, args, rank, world, local_rank, device):
     X, y, w_true = synthetic_glm_shard(rows, 256, seed=100 + rank, device=device)
     if impl == "b200":
         glm = FederatedGLM(X, y, rank, world, lr=2.0)
-        step = glm.step
+        step, coef = glm.step, glm.w
     else:       # comparator: two cuBLAS GEMVs + elementwise + ncclAllReduce of the 259-float payload
-        w = torch.zeros(257, device=device)
+        w = coef = torch.zeros(257, device=device)
 
         def step():
             z = (X @ w[:256].to(X.dtype)).float() + w[256]
@@ -253,6 +277,8 @@ def run_glm_arm(impl, args, rank, world, local_rank, device):
             loss = step()
         ms = max_over_ranks(t.stop(), device)
         launches = LAUNCHES[0] - l0
+    if args.dump_outputs and impl == args.impl and rank == 0:
+        dump_outputs(args.dump_outputs, {"loss": loss, "coefficients": coef})
     t0 = time.perf_counter()
     for _ in range(iters):
         lv = float(step().item())                  # end to end: the iteration's loss is read back every iteration

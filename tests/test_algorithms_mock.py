@@ -145,6 +145,45 @@ def test_bench_reference_arm_reports_unavailable():
     assert d["impl"] == "reference" and "unavailable" in d
 
 
+def test_bench_dump_samples_large_outputs_at_fixed_indices(tmp_path, monkeypatch):
+    import torch
+
+    sys.path.insert(0, ROOT)
+    import bench
+
+    monkeypatch.setattr(bench, "DUMP_MAX_ELEMS", 1000)
+    x = torch.arange(5000, dtype=torch.float64)
+    bench.dump_outputs(str(tmp_path / "a"), {"loss": torch.tensor(2.5), "global_model": x})
+    bench.dump_outputs(str(tmp_path / "b"), {"global_model": x.clone()})
+    loss, a, b = (np.load(tmp_path / p) for p in ("a/loss.npy", "a/global_model.npy", "b/global_model.npy"))
+    assert loss.dtype == np.float32 and loss.shape == () and loss == 2.5
+    assert a.dtype == np.float32 and a.shape == (1000,) and (a == b).all() and (np.diff(a) > 0).all()
+
+
+@pytest.mark.gpu
+def test_bench_dumps_the_last_timed_round(tmp_path):
+    """--steps sets the timed rounds; --dump-outputs writes their last result, and the same arguments give the same inputs
+    and so the same dump on every run (what makes two builds comparable output for output).  resnet_mini is the flagship's
+    path at 64x64 images -- every convolution on the project's kernels; resnet_tiny's narrow layers fall back to cuDNN,
+    whose autotuned algorithm choice may differ between runs."""
+    runs = []
+    for k in range(2):
+        out = tmp_path / f"outputs{k}"
+        p = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--model", "resnet_mini", "--steps", "2", "--warmup", "1",
+                            "--no-e2e", "--baselines", "", "--dump-outputs", str(out)], capture_output=True, text=True, timeout=600)
+        assert p.returncode == 0, p.stderr[-3000:]
+        d = json.loads(p.stdout.strip().splitlines()[-1])
+        assert d["steps"] == 2 and sorted(f.name for f in out.iterdir()) == ["global_model.npy", "loss.npy"]
+        loss, model = np.load(out / "loss.npy"), np.load(out / "global_model.npy")
+        assert loss.dtype == np.float32 and float(loss) == d["final_loss"]
+        assert model.dtype == np.float32 and model.shape == (min(d["config"]["n_federated_params"], 1 << 23),)
+        assert np.isfinite(model).all()
+        runs.append((loss, model))
+    (l0, m0), (l1, m1) = runs
+    np.testing.assert_allclose(l1, l0, rtol=1e-5)
+    np.testing.assert_allclose(m1, m0, rtol=1e-5, atol=1e-6 * float(np.abs(m0).max()))
+
+
 def test_graft_entry_build_is_incremental():
     sys.path.insert(0, ROOT)
     import __graft_entry__ as g

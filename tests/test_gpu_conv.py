@@ -118,6 +118,27 @@ def test_conv_wgrad_accumulates_into_fp32(dev, n, cin, cout, h, w, k, stride, pa
     torch.testing.assert_close(dw - base, ref, rtol=1e-3, atol=2e-3 * float(ref.abs().max()))
 
 
+@pytest.mark.parametrize("cin,cout,k,splits", [(64, 64, 1, 0), (64, 64, 3, 0), (256, 128, 3, 0), (64, 64, 1, 37)])
+def test_split_wgrad_is_the_same_sum_every_run(dev, cin, cout, k, splits):
+    """A filter gradient whose K (the pixels) is split over many CTAs: the partial tiles are added in a fixed order, so
+    repeated launches give bit-identical results (and still the right ones)."""
+    from vantage6_b200.ops import conv as C
+    from vantage6_b200.ops import native
+
+    n, hw, pad = 32, 56, k // 2
+    assert native().conv_wgrad_workspace(n, hw, hw, cin, cout, k, k, 1, pad, splits) > 0
+    x, dy = _t((n, cin, hw, hw), 11), _t((n, cout, hw, hw), 12, 0.1)
+    base = torch.randn((cout, k, k, cin), device=dev)
+    outs = []
+    for _ in range(3):
+        dw = base.clone()
+        C.conv_wgrad(dy, x, dw, (k, k), 1, pad, splits=splits)
+        outs.append(dw)
+    assert all(torch.equal(outs[0], o) for o in outs[1:])
+    ref = torch.nn.grad.conv2d_weight(x.float(), (cout, cin, k, k), dy.float(), padding=pad).permute(0, 2, 3, 1)
+    torch.testing.assert_close(outs[0] - base, ref, rtol=1e-3, atol=2e-3 * float(ref.abs().max()))
+
+
 def test_resnet_bottleneck_tc_path_matches_cudnn_path(dev, monkeypatch):
     """A ResNet stage through FederatedTrainer-style flat buffers: V6B200_CONV=tc (own kernels, statistics in the
     convolution epilogue, filter gradients straight into the flat buffer) vs V6B200_CONV=cudnn (round-1 path)."""

@@ -33,6 +33,10 @@ def network(tmp_path_factory):
         pd.DataFrame({"age": rng.normal(55 + 10 * i, 8, n).round(1), "sex": rng.choice(["f", "m"], n)}).to_csv(home / f"patients{i}.csv", index=False)
         dbs.append({"default": str(p), "patients": str(home / f"patients{i}.csv")})
     old = os.environ.get("V6B200_HOME")
+    # CPU nodes on any machine: the node processes (and the algorithms they start) inherit this environment, and on a GPU
+    # box they would otherwise all pick up device 0 -- two NCCL ranks on one GPU
+    cpu_only = pytest.MonkeyPatch()
+    cpu_only.setenv("CUDA_VISIBLE_DEVICES", "")
     net = DemoNetwork(2, home=str(home), databases=dbs)
     try:
         net.start()
@@ -40,6 +44,7 @@ def network(tmp_path_factory):
         yield net
     finally:
         net.stop()
+        cpu_only.undo()
         if old is None:
             os.environ.pop("V6B200_HOME", None)
         else:

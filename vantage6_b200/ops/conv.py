@@ -121,6 +121,17 @@ def conv_dgrad(dy: torch.Tensor, w: torch.Tensor, in_hw: Tuple[int, int], pad: i
     return dx
 
 
+def _wgrad(dy, x, dw, n, h, w, cin, cout, r, s, stride, pad, scale, splits, force_im2col, pitches=(0, 0, 0)) -> None:
+    """One WGRAD launch.  When a tile's K is split into several ranges, their partial tiles go to a workspace (allocated here, on
+    the current stream) and a second kernel adds them into ``dw`` in one fixed order: the same sum on every run."""
+    C = native()
+    ws_floats = C.conv_wgrad_workspace(n, h, w, cin, cout, r, s, stride, pad, int(splits))
+    ws = torch.empty(ws_floats, device=dw.device, dtype=torch.float32) if ws_floats else None
+    count(2 if ws_floats else 1)
+    C.conv_wgrad(dy.data_ptr(), x.data_ptr(), dw.data_ptr(), n, h, w, cin, cout, r, s, stride, pad, float(scale), int(splits), force_im2col,
+                 stream_ptr(), *pitches, 0 if ws is None else ws.data_ptr(), ws_floats)
+
+
 def conv_wgrad(dy: torch.Tensor, x: torch.Tensor, dw: torch.Tensor, rs: Tuple[int, int], stride: int = 1, pad: int = 0,
                scale: float = 1.0, splits: int = 0, force_im2col: bool = False) -> torch.Tensor:
     """``dw`` (fp32, memory [Cout, R, S, Cin], e.g. the ``.grad`` view of a flat model) ``+= scale * dy^T . im2col(x)``."""
@@ -130,9 +141,7 @@ def conv_wgrad(dy: torch.Tensor, x: torch.Tensor, dw: torch.Tensor, rs: Tuple[in
     cout = dy.shape[1]
     r, s = rs
     assert dw.numel() == cout * r * s * cin
-    count(1)
-    native().conv_wgrad(dy.data_ptr(), x.data_ptr(), dw.data_ptr(), n, h, wd, cin, cout, r, s, stride, pad, float(scale), int(splits),
-                        force_im2col, stream_ptr(), 0, 0, 0)
+    _wgrad(dy, x, dw, n, h, wd, cin, cout, r, s, stride, pad, scale, splits, force_im2col)
     return dw
 
 
@@ -167,9 +176,7 @@ def stem_wgrad(dy: torch.Tensor, xs: torch.Tensor, dws: torch.Tensor) -> torch.T
     n, c16, hs, wsz = xs.shape
     cout = dy.shape[1]
     assert dws.dtype == torch.float32 and dws.numel() == cout * 256
-    count(1)
-    native().conv_wgrad(dy.data_ptr(), xs.data_ptr(), dws.data_ptr(), n, hs, wsz - 3, 64, cout, 4, 1, 1, 0, 1.0, 0, True, stream_ptr(),
-                        32, wsz * 32, hs * wsz * 32)
+    _wgrad(dy, xs, dws, n, hs, wsz - 3, 64, cout, 4, 1, 1, 0, 1.0, 0, True, (32, wsz * 32, hs * wsz * 32))
     return dws
 
 
@@ -217,6 +224,5 @@ def linear_wgrad(dy: torch.Tensor, x: torch.Tensor, dw: torch.Tensor, scale: flo
     m, n = dy.shape
     m2, k = x.shape
     assert m == m2 and dw.numel() == n * k
-    count(1)
-    native().conv_wgrad(dy.data_ptr(), x.data_ptr(), dw.data_ptr(), 1, 1, m, k, n, 1, 1, 1, 0, float(scale), 0, False, stream_ptr(), 0, 0, 0)
+    _wgrad(dy, x, dw, 1, 1, m, k, n, 1, 1, 1, 0, scale, 0, False)
     return dw

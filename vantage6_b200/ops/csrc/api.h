@@ -207,7 +207,8 @@ int v6_conv_dgrad(const void* dy, const void* w, void* dx, int N, int H, int W, 
                   int red_accumulate, float* scratch, cudaStream_t stream);
 int v6_conv_wgrad(const void* dy, const void* x, float* dw, int N, int H, int W, int Cin, int Cout, int R, int S, int stride, int pad,
                   float scale, int splits, int force_im2col, long long pitch_w, long long pitch_h, long long pitch_n,
-                  cudaStream_t stream);
+                  float* ws, long long ws_floats, cudaStream_t stream);
+long long v6_conv_wgrad_workspace(int N, int H, int W, int Cin, int Cout, int R, int S, int stride, int pad, int splits);
 #ifdef __cplusplus
 }
 #endif

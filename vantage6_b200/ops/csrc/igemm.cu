@@ -28,7 +28,10 @@
 // ALL row tiles of the CTA (a CTA keeps one column block), published once with fp64 reductions into L2; the last CTA
 // of a column block to arrive does the per-channel finalize (mean, rstd, scale/bias, running statistics) from the
 // totals.  The separate statistics pass over Y (bn.cu::bn_stats_kernel) disappears.
-// WGRAD epilogue = red.global.add.v4.f32 of the fp32 accumulators into dW (split-K partial sums meet in L2).
+// WGRAD epilogue = the fp32 accumulators added into dW when a tile has one k-range; with several, every k-range stores its
+// partial tile into its own workspace slice and wgrad_split_sum_kernel adds the slices into dW in one fixed order -- the
+// same sum on every run (reductions in L2 would add them in arrival order).  Without it two runs of the same training
+// drift apart within a few rounds and outputs of two builds cannot be compared.
 #include <cuda.h>
 #include <math.h>
 #include <stdlib.h>
@@ -92,6 +95,7 @@ struct Params {
     __nv_bfloat16* dx;
     // WGRAD
     float* dw; long long ldw; int splits, kb_per_split; float out_scale;
+    float* ws;                       // splits > 1: [splits][M][ldw] partial tiles, one slice per k-range
     // FPROP BatchNorm statistics (null gamma -> off)
     const float* gamma; const float* beta; float* running_mean; float* running_var; long long* num_batches_tracked;
     float* mean_out; float* rstd_out; float* scale_out; float* bias_out;
@@ -136,9 +140,6 @@ V6_DEVINL void tma_load_2d_u(uint32_t smem_dst, const void* tmap, uint32_t bar, 
 V6_DEVINL void tma_load_3d_u(uint32_t smem_dst, const void* tmap, uint32_t bar, int c0, int c1, int c2) {
     asm volatile("cp.async.bulk.tensor.3d.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4, %5}], [%2];"
                  :: "r"(smem_dst), "l"(tmap), "r"(bar), "r"(c0), "r"(c1), "r"(c2) : "memory");
-}
-V6_DEVINL void red_add_f4(float* p, float a, float b, float c, float d) {
-    asm volatile("red.global.add.v4.f32 [%0], {%1,%2,%3,%4};" :: "l"(p), "f"(a), "f"(b), "f"(c), "f"(d) : "memory");
 }
 // explicit shared-state-space accesses for the epilogue's staging boxes (through generic pointers the compiler emitted
 // LD.E / ST.E -- generic-address loads with global-memory-like latency, profiles/ncu_igemm_r2c.md)
@@ -571,14 +572,15 @@ igemm_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_constant__
             tcgen05_fence_after();
             const uint32_t t_row = tmem_base + acc * 256 + ((uint32_t)(quad * 32) << 16);
             if (MODE == WGRAD) {
-                // fp32 accumulators -> dW[row][n_blk*block_n + col] (+=); row = output channel.  split-K partial sums meet by
-                // red.add in L2; with ONE k-range per tile the tile owns its output and a plain load-add-store does it -- L2 fp32
-                // reductions run at ~0.7 TB/s, an order of magnitude below plain stores, and were the whole gap to cuDNN on the
-                // layers with large filters (512x512x3x3: 19 MB of reductions per launch; profiles/kernel_bench_linear_bwd_r2.txt)
+                // fp32 accumulators -> dW[row][n_blk*block_n + col] (+=); row = output channel.  With ONE k-range per tile the
+                // tile owns its output and a plain load-add-store does it; with several, this k-range's partial tile goes to its
+                // workspace slice with plain stores (wgrad_split_sum_kernel adds the slices in a fixed order) -- no L2 reductions, which
+                // run at ~0.7 TB/s, an order of magnitude below plain stores (profiles/kernel_bench_linear_bwd_r2.txt)
                 const int row = it.m_blk * BLOCK_M + quad * 32 + lane;
                 const int ncols = wgrad_chunks(it.n_blk) * 64;
-                float* drow = P.dw + (long long)row * P.ldw + it.n_blk * P.block_n;
                 const bool owned = P.splits == 1;
+                float* drow = (owned ? P.dw : P.ws + (long long)(it.kb0 / P.kb_per_split) * P.M * P.ldw)
+                              + (long long)row * P.ldw + it.n_blk * P.block_n;
 #pragma unroll 1
                 for (int c = half * 32; c < ncols; c += 64) {
                     uint32_t v[32];
@@ -598,8 +600,9 @@ igemm_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_constant__
                         } else {
 #pragma unroll
                             for (int j = 0; j < 32; j += 4)
-                                red_add_f4(drow + c + j, __uint_as_float(v[j]) * P.out_scale, __uint_as_float(v[j + 1]) * P.out_scale,
-                                           __uint_as_float(v[j + 2]) * P.out_scale, __uint_as_float(v[j + 3]) * P.out_scale);
+                                *reinterpret_cast<float4*>(drow + c + j) = make_float4(
+                                    __uint_as_float(v[j]) * P.out_scale, __uint_as_float(v[j + 1]) * P.out_scale,
+                                    __uint_as_float(v[j + 2]) * P.out_scale, __uint_as_float(v[j + 3]) * P.out_scale);
                         }
                     }
                 }
@@ -984,26 +987,23 @@ extern "C" int v6_conv_dgrad(const void* dy, const void* w, void* dx, int N, int
     return launch(DGRAD, ta, tb, tc, P, stream);
 }
 
-// dw[Cout,R,S,Cin] (fp32) += scale * dy[N,P,Q,Cout]^T . im2col(x[N,H,W,Cin])
-extern "C" int v6_conv_wgrad(const void* dy, const void* x, float* dw, int N, int H, int W, int Cin, int Cout, int R, int S, int stride,
-                             int pad, float scale, int splits, int force_im2col, long long pitch_w, long long pitch_h, long long pitch_n,
-                             cudaStream_t stream) {
-    using namespace igemm;
+namespace {
+// The GEMM shape of a WGRAD launch and its plan (N tile, k-ranges per tile); shared by the launch and its workspace query.
+int wgrad_shape(igemm::Params& P, int N, int H, int W, int Cin, int Cout, int R, int S, int stride, int pad, int splits) {
     if (Cin % 64 != 0 || Cout % 8 != 0 || (R != S && pad != 0)) return (int)cudaErrorInvalidValue;
     const int Pp = (H + 2 * pad - R) / stride + 1, Qq = (W + 2 * pad - S) / stride + 1;
     const long long pix = (long long)N * Pp * Qq;
     if (pix >= (1LL << 31)) return (int)cudaErrorInvalidValue;
-    const bool plain = R == 1 && S == 1 && stride == 1 && pad == 0 && !force_im2col && !pitch_w;
-    Params P = {};
     P.M = Cout; P.N = R * S * Cin; P.num_kb = (int)((pix + 63) / 64); P.block_n = 256;
-    P.b_im2col = plain ? 0 : 1; P.PQ = Pp * Qq; P.Q = Qq; P.stride = stride; P.pad = pad; P.S = S; P.cblocks = Cin / 64; P.taps = R * S;
-    P.dw = dw; P.ldw = (long long)R * S * Cin; P.out_scale = scale;
+    P.PQ = Pp * Qq; P.Q = Qq; P.stride = stride; P.pad = pad; P.S = S; P.cblocks = Cin / 64; P.taps = R * S;
     if (splits <= 0) {
         // (N tile, k-ranges per tile) by a small cost model in cycles: waves x k-blocks x max(MMA, operand fetch through L2) for the
-        // main loop; the epilogue moves Cout x R*S*Cin x 4 B per k-range -- through L2 reductions (~370 B/cycle chip-wide, measured)
-        // when a tile has several k-ranges, by plain load-add-store (~3000 B/cycle) when it has one.  Few tiles + long K (the
+        // main loop; the epilogue moves Cout x R*S*Cin x 4 B by plain load-add-store (~3000 B/cycle) when a tile has one k-range;
+        // with several, each k-range stores its partial and the ordered sum reads them all back and updates dW (priced at the
+        // same plain-memory rate, not measured separately).  Few tiles + long K (the
         // 56x56 layers) -> many k-ranges of a tiny output; big filters + short K (7x7 / 14x14 layers, nn.Linear) -> one k-range.
-        // MEASURED: the model's plan is slower than the simple one below (about one wave of items, 256-column tiles, reductions):
+        // MEASURED while split tiles were still summed by L2 reductions (~370 B/cycle): the model's plan was slower than the simple one
+        // below (about one wave of items, 256-column tiles):
         // nn.Linear 768 -> 3072 at 4096 tokens 38 vs 27 us, ResNet-50 round 51.5 vs 50.4 ms, BERT-base 31.4 vs 30.0 ms -- the
         // owned-tile load-add-store epilogue (32 rows x 16 B per instruction, 1 KB apart) and the longer per-CTA K loop cost more than
         // the reductions they avoid.  Kept behind V6B200_WGRAD_PLAN=1 with its tests.
@@ -1019,7 +1019,7 @@ extern "C" int v6_conv_wgrad(const void* dy, const void* x, float* dw, int N, in
                 const long long items = tiles * s;
                 const double waves = (double)((items + 147) / 148);
                 const double kb = (double)((P.num_kb + s - 1) / s);
-                const double t = waves * (kb * per_kb + 1500.0) + (s == 1 ? out_bytes / 3000.0 : out_bytes * s / 370.0);
+                const double t = waves * (kb * per_kb + 1500.0) + (s == 1 ? out_bytes / 3000.0 : out_bytes * (2.0 * s + 2.0) / 3000.0);
                 if (t < best) { best = t; best_bn = bn; best_s = s; }
             }
         }
@@ -1036,10 +1036,83 @@ extern "C" int v6_conv_wgrad(const void* dy, const void* x, float* dw, int N, in
     if (splits > P.num_kb) splits = P.num_kb;
     P.kb_per_split = (P.num_kb + splits - 1) / splits;
     P.splits = (P.num_kb + P.kb_per_split - 1) / P.kb_per_split;
+    return 0;
+}
+
+// dW += the partial tiles of a WGRAD with several k-ranges per tile, in a fixed order.  A block covers 256 / groups consecutive
+// float4s; thread group g sums the slices g, g + groups, ... (four loads in flight) and group 0 adds the group sums in group order.
+__global__ void __launch_bounds__(256) wgrad_split_sum_kernel(const float4* __restrict__ ws, float4* __restrict__ dw, long long count4,
+                                                              int splits, int groups) {
+    __shared__ float4 part[256];
+    const int per = 256 / groups, e = threadIdx.x % per, g = threadIdx.x / per;
+    auto add = [](float4& a, const float4& v) { a.x += v.x; a.y += v.y; a.z += v.z; a.w += v.w; };
+    for (long long base = (long long)blockIdx.x * per; base < count4; base += (long long)gridDim.x * per) {
+        const long long i = base + e;
+        float4 acc = make_float4(0.f, 0.f, 0.f, 0.f);
+        if (i < count4) {
+            int sp = g;
+            for (; sp + 3 * groups < splits; sp += 4 * groups) {
+                float4 v[4];
+#pragma unroll
+                for (int u = 0; u < 4; ++u) v[u] = __ldcs(ws + (long long)(sp + u * groups) * count4 + i);
+#pragma unroll
+                for (int u = 0; u < 4; ++u) add(acc, v[u]);
+            }
+            for (; sp < splits; sp += groups) add(acc, __ldcs(ws + (long long)sp * count4 + i));
+        }
+        part[threadIdx.x] = acc;
+        __syncthreads();
+        if (g == 0 && i < count4) {
+            float4 sum = part[e];
+            for (int k = 1; k < groups; ++k) add(sum, part[k * per + e]);
+            float4 d = dw[i];
+            add(d, sum);
+            dw[i] = d;
+        }
+        __syncthreads();
+    }
+}
+}  // namespace
+
+// floats of workspace v6_conv_wgrad needs for this problem (0: one k-range per tile, no workspace)
+extern "C" long long v6_conv_wgrad_workspace(int N, int H, int W, int Cin, int Cout, int R, int S, int stride, int pad, int splits) {
+    igemm::Params P = {};
+    if (wgrad_shape(P, N, H, W, Cin, Cout, R, S, stride, pad, splits)) return 0;
+    return P.splits > 1 ? (long long)P.splits * P.M * P.N : 0;
+}
+
+// dw[Cout,R,S,Cin] (fp32) += scale * dy[N,P,Q,Cout]^T . im2col(x[N,H,W,Cin]); ws: v6_conv_wgrad_workspace floats (the k-range partials)
+extern "C" int v6_conv_wgrad(const void* dy, const void* x, float* dw, int N, int H, int W, int Cin, int Cout, int R, int S, int stride,
+                             int pad, float scale, int splits, int force_im2col, long long pitch_w, long long pitch_h, long long pitch_n,
+                             float* ws, long long ws_floats, cudaStream_t stream) {
+    using namespace igemm;
+    Params P = {};
+    const int rc = wgrad_shape(P, N, H, W, Cin, Cout, R, S, stride, pad, splits);
+    if (rc) return rc;
+    const long long pix = (long long)N * P.PQ;
+    const bool plain = R == 1 && S == 1 && stride == 1 && pad == 0 && !force_im2col && !pitch_w;
+    P.b_im2col = plain ? 0 : 1;
+    P.dw = dw; P.ldw = (long long)R * S * Cin; P.out_scale = scale;
+    const long long count = (long long)P.M * P.N;
+    if (P.splits > 1) {
+        if (ws == nullptr || ws_floats < P.splits * count) return (int)cudaErrorInvalidValue;
+        P.ws = ws;
+    }
     alignas(64) CUtensorMap ta, tb, tc;
     if (v6_make_tmap_2d_bf16(&ta, (uint64_t)dy, (uint64_t)pix, Cout, (uint64_t)Cout * 2, 64, 64, 1)) return -2;
     if (plain) { if (v6_make_tmap_2d_bf16(&tb, (uint64_t)x, (uint64_t)pix, Cin, (uint64_t)Cin * 2, 64, 64, 1)) return -2; }
-    else { ConvGeom g{N, H, W, Cin, R, S, stride, pad, Pp, Qq, pitch_w, pitch_h, pitch_n}; if (im2col_map(&tb, x, g, 64)) return -2; }
+    else { ConvGeom g{N, H, W, Cin, R, S, stride, pad, P.PQ / P.Q, P.Q, pitch_w, pitch_h, pitch_n}; if (im2col_map(&tb, x, g, 64)) return -2; }
     tc = ta;
-    return launch(WGRAD, ta, tb, tc, P, stream);
+    const int lrc = launch(WGRAD, ta, tb, tc, P, stream);
+    if (lrc || P.splits == 1) return lrc;
+    // enough (element, slice group) threads to fill the GPU: many slices of a small filter are summed by up to 32 groups
+    const long long count4 = count / 4;                  // R*S*Cin is a multiple of 64
+    int groups = 1;
+    while (groups < 32 && groups * 2 <= P.splits && count4 * groups < 148LL * 2048) groups *= 2;
+    const int per = 256 / groups;
+    const long long blocks = (count4 + per - 1) / per;
+    wgrad_split_sum_kernel<<<(unsigned)(blocks < 148 * 8 ? blocks : 148 * 8), 256, 0, stream>>>(
+        reinterpret_cast<const float4*>(ws), reinterpret_cast<float4*>(dw), count4, P.splits, groups);
+    V6_CHECK_LAUNCH();
+    return 0;
 }

@@ -283,10 +283,12 @@ PYBIND11_MODULE(_C, m) {
                             P<float>(red_dbeta), P<float>(red_coef), red_accumulate ? 1 : 0, P<float>(scratch), S(s)), "conv_dgrad");
     });
     m.def("conv_wgrad", [](u64 dy, u64 x, u64 dw, int N, int H, int W, int Cin, int Cout, int R, int Sw, int stride, int pad,
-                           float scale, int splits, bool force_im2col, u64 s, long long pitch_w, long long pitch_h, long long pitch_n) {
+                           float scale, int splits, bool force_im2col, u64 s, long long pitch_w, long long pitch_h, long long pitch_n,
+                           u64 ws, long long ws_floats) {
         check(v6_conv_wgrad(P<void>(dy), P<void>(x), P<float>(dw), N, H, W, Cin, Cout, R, Sw, stride, pad, scale, splits,
-                            force_im2col, pitch_w, pitch_h, pitch_n, S(s)), "conv_wgrad");
+                            force_im2col, pitch_w, pitch_h, pitch_n, P<float>(ws), ws_floats, S(s)), "conv_wgrad");
     });
+    m.def("conv_wgrad_workspace", &v6_conv_wgrad_workspace);
     // ------------------------------------------------------------------ K1 / tcgen05 GEMM
     m.def("gemm_bf16", [](u64 A, u64 B, u64 C, u64 bias, int M, int N, int K, int lda, int ldb, int ldc, int act, u64 s) {
         check(v6_gemm_bf16(P<void>(A), P<void>(B), P<void>(C), P<float>(bias), M, N, K, lda, ldb, ldc, act, S(s)), "gemm_bf16");
