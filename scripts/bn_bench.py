@@ -1,16 +1,13 @@
-"""Bandwidth of the BatchNorm passes on the ResNet-50 layer shapes (batch 64), per tuning variant.
+"""Bandwidth of the BatchNorm passes on the ResNet-50 layer shapes (batch 64).
 
     PYTHONPATH=. python scripts/bn_bench.py [--out gpurun_out/bn_bench.jsonl]
 
-Runs itself once per V6B200_BN_CFG value (the variant is read once per process) and prints, per layer shape, the time of
-every pass (statistics, apply, backward reduce, backward apply), the bytes it has to move and the resulting GB/s next to
-the measured copy bandwidth of the box (MEASURED_PEAKS.json).  Buffers rotate over enough copies to exceed the 126 MB L2.
+Prints, per layer shape, the time of every pass (statistics, apply, backward reduce, backward apply), the bytes it has to
+move and the resulting GB/s next to the measured copy bandwidth of the box (MEASURED_PEAKS.json).  Buffers rotate over
+enough copies to exceed the 126 MB L2.
 """
 import argparse
 import json
-import os
-import subprocess
-import sys
 
 SHAPES = [  # (H=W, C, relu, residual, how many per forward pass)
     (112, 64, True, False, 1),
@@ -21,7 +18,7 @@ SHAPES = [  # (H=W, C, relu, residual, how many per forward pass)
 ]
 
 
-def child(cfg: str):
+def bench():
     import torch
 
     from vantage6_b200.ops import native, stream_ptr
@@ -44,6 +41,7 @@ def child(cfg: str):
         return e0.elapsed_time(e1) / iters * 1e3        # us
 
     tot = {"stats": 0.0, "apply": 0.0, "bwd_reduce+apply": 0.0}
+    lines = []
     for (hw, C, relu, res, mult) in SHAPES:
         R = N * hw * hw
         nbytes = R * C * 2
@@ -76,35 +74,24 @@ def child(cfg: str):
         mb = nbytes / 8 if relu else 0
         b_apply = nbytes * (2 + (1 if res else 0)) + mb
         b_bwd = (2 * nbytes + mb) * 2 + nbytes * (1 + (1 if res else 0))
-        rec = dict(cfg=cfg, hw=hw, C=C, relu=relu, res=res, mult=mult, mb_per_tensor=nbytes / 1e6, stats_us=t_fwd - t_apply, apply_us=t_apply,
+        rec = dict(hw=hw, C=C, relu=relu, res=res, mult=mult, mb_per_tensor=nbytes / 1e6, stats_us=t_fwd - t_apply, apply_us=t_apply,
                    apply_gbs=b_apply / t_apply * 1e-3, stats_gbs=nbytes / max(t_fwd - t_apply, 1e-3) * 1e-3, bwd_us=t_bwd, bwd_gbs=b_bwd / t_bwd * 1e-3)
         print(json.dumps(rec), flush=True)
+        lines.append(json.dumps(rec))
         tot["stats"] += mult * (t_fwd - t_apply)
         tot["apply"] += mult * t_apply
         tot["bwd_reduce+apply"] += mult * t_bwd
         del x, dy, y, dx, rs, dres, mask
-    print(json.dumps(dict(cfg=cfg, per_step_ms={k: v / 1e3 for k, v in tot.items()})), flush=True)
+    lines.append(json.dumps(dict(per_step_ms={k: v / 1e3 for k, v in tot.items()})))
+    print(lines[-1], flush=True)
+    return lines
 
 
 def main():
     ap = argparse.ArgumentParser()
-    ap.add_argument("--cfgs", default="0,1,2")
     ap.add_argument("--out", default="")
-    ap.add_argument("--child", default="")
     a = ap.parse_args()
-    if a.child:
-        child(a.child)
-        return
-    lines = []
-    for cfg in a.cfgs.split(","):
-        env = dict(os.environ, V6B200_BN_CFG=cfg)
-        pr = subprocess.run([sys.executable, __file__, "--child", cfg], env=env, stdout=subprocess.PIPE, stderr=subprocess.PIPE, text=True, timeout=300)
-        for ln in pr.stdout.splitlines():
-            if ln.startswith("{"):
-                lines.append(ln)
-                print(ln)
-        if pr.returncode != 0:
-            print(f"# cfg {cfg} failed rc={pr.returncode}: {pr.stderr[-500:]}")
+    lines = bench()
     if a.out:
         with open(a.out, "w") as f:
             f.write("\n".join(lines) + "\n")

@@ -234,83 +234,3 @@ def test_side_stream_filter_gradients_match_inline(dev, monkeypatch):
     g.replay()
     torch.cuda.synchronize()
     torch.testing.assert_close(fm.grad, g_inline, rtol=1e-3, atol=1e-5 * float(g_inline.abs().max()) + 1e-7)
-
-
-def test_bn_backward_reduction_in_dgrad_epilogue_matches_separate_pass(dev, monkeypatch):
-    """EPI_RED (csrc/igemm.cu): the data-gradient kernel of the consuming convolution also produces the BatchNorm backward's
-    per-channel sums / coefficients / dgamma / dbeta; against the same model with the reduction as its own pass."""
-    from vantage6_b200.models.flat import FlatModel
-    from vantage6_b200.models.resnet import Bottleneck
-    from vantage6_b200.models.transformer import attach_shadow
-    from vantage6_b200.ops import bn as BN
-
-    monkeypatch.setenv("V6B200_CONV", "tc")
-
-    def _down(cin, cout, stride):
-        from vantage6_b200.models.conv import ShadowConv2d
-        from vantage6_b200.ops.bn import FusedBatchNormAct
-
-        return torch.nn.Sequential(ShadowConv2d(cin, cout, 1, stride=stride, bias=False), FusedBatchNormAct(cout, relu=False))
-
-    def run(flag):
-        monkeypatch.setenv("V6B200_BN_RED", flag)
-        torch.manual_seed(0)
-        m = torch.nn.Sequential(Bottleneck(64, 64, 1, _down(64, 256, 1)), Bottleneck(256, 64), Bottleneck(256, 64)).to(dev).to(memory_format=torch.channels_last)
-        for mod in m.modules():
-            if isinstance(mod, Bottleneck):
-                torch.nn.init.normal_(mod.bn3.weight, 1.0, 0.1)
-        fm = FlatModel(m, shadow=None)
-        fm.shadow = fm.flat.to(torch.bfloat16)
-        attach_shadow(m, fm)
-        m.train()
-        x = _t((8, 64, 28, 28), 3).requires_grad_()
-        fm.zero_grad()
-        (m(x).float() ** 2).mean().backward()
-        fm.flush_grad_sink()
-        torch.cuda.synchronize()
-        bn_g = torch.cat([p.grad.flatten() for n, p in m.named_parameters() if "bn" in n or "downsample.1" in n])
-        return x.grad.float().clone(), fm.grad.clone(), bn_g.clone()
-
-    from vantage6_b200.ops import LAUNCHES
-
-    l0 = LAUNCHES[0]
-    dx1, g1, b1 = run("1")
-    n_fused = LAUNCHES[0] - l0
-    l0 = LAUNCHES[0]
-    dx0, g0, b0 = run("0")
-    n_sep = LAUNCHES[0] - l0
-    assert n_fused < n_sep, (n_fused, n_sep)                  # 8 of the 10 BatchNorm backward reductions ride in a dgrad epilogue
-    torch.testing.assert_close(b1, b0, rtol=2e-3, atol=2e-3 * float(b0.abs().max()))
-    assert torch.nn.functional.cosine_similarity(dx1.flatten(), dx0.flatten(), dim=0) > 0.9999
-    torch.testing.assert_close(dx1, dx0, rtol=2e-2, atol=2e-2 * float(dx0.abs().max()))
-    assert torch.nn.functional.cosine_similarity(g1, g0, dim=0) > 0.9999
-
-
-@pytest.mark.parametrize("n,cin,cout,hw,r", [(4, 64, 64, 16, 1), (2, 128, 64, 16, 3), (4, 256, 64, 8, 1)])
-def test_dgrad_epilogue_bn_reduction_unit(dev, n, cin, cout, hw, r):
-    """EPI_RED in isolation: dx unchanged, dgamma / dbeta / coefficients equal to the formulas of the separate reduction pass."""
-    from vantage6_b200.ops import conv as C
-
-    pad = 1 if r == 3 else 0
-    dy = _t((n, cout, hw, hw), 1)
-    w = (_t((cout, cin, r, r), 2) * (1.0 / (cout * r * r) ** 0.5)).contiguous(memory_format=torch.channels_last)
-    xbn = _t((n, cin, hw, hw), 3)
-    R = n * hw * hw
-    mask_bits = torch.rand(R, cin, device=dev) > 0.4
-    mask = (mask_bits.view(R, cin // 8, 8).to(torch.uint8) << torch.arange(8, device=dev, dtype=torch.uint8)).sum(-1).to(torch.uint8)
-    mean, rstd, gamma = torch.randn(cin, device=dev) * 0.1, torch.rand(cin, device=dev) + 0.5, torch.rand(cin, device=dev) + 0.5
-    dgamma, dbeta, coef = torch.zeros(cin, device=dev), torch.zeros(cin, device=dev), torch.zeros(3 * cin, device=dev)
-    ref_dx = C.conv_dgrad(dy, w, (hw, hw), pad)
-    dx = C.conv_dgrad(dy, w, (hw, hw), pad, bn_red=dict(x=xbn, mask=mask, mean=mean, rstd=rstd, gamma=gamma, dgamma=dgamma, dbeta=dbeta,
-                                                         coef=coef, accumulate=False))
-    torch.cuda.synchronize()
-    torch.testing.assert_close(dx.float(), ref_dx.float(), rtol=0, atol=0)
-    g = dx.float().permute(0, 2, 3, 1).reshape(R, cin) * mask_bits
-    xh = (xbn.float().permute(0, 2, 3, 1).reshape(R, cin) - mean) * rstd
-    tg, tgx = g.sum(0), (g * xh).sum(0)
-    torch.testing.assert_close(dbeta, tg, rtol=2e-3, atol=2e-3 * float(tg.abs().max()))
-    torch.testing.assert_close(dgamma, tgx, rtol=2e-3, atol=2e-3 * float(tgx.abs().max()))
-    k0 = gamma * rstd
-    k1 = -k0 * rstd * tgx / R
-    k2 = -k0 * tg / R - k1 * mean
-    torch.testing.assert_close(coef, torch.cat([k0, k1, k2]), rtol=2e-3, atol=2e-3 * float(k0.abs().max()))

@@ -156,8 +156,9 @@ def test_stem_space_to_depth_matches_direct_conv(dev, N, H, W, O):
 
 
 @pytest.mark.parametrize("N,C,H,W", [(4, 64, 112, 112), (2, 64, 10, 14), (3, 128, 16, 16)])
-def test_fused_bn_relu_maxpool_matches_separate_passes(dev, N, C, H, W):
-    """Stem: maxpool(relu(bn(x))) as one pass per direction (csrc/bn.cu) against the separate fused-BN + max-pool kernels."""
+def test_stem_bn_apply_maxpool_matches_torch(dev, N, C, H, W):
+    """Stem tail: BatchNorm apply + ReLU with the statistics of the producing convolution (``apply_pre``), then the 3x3 / s2
+    max-pool, against ``max_pool2d(relu(x * scale + bias))`` in fp32 PyTorch: the output, dx, dgamma and dbeta."""
     from vantage6_b200.ops import bn as BN
     from vantage6_b200.ops.pool import MaxPool3x3s2
 
@@ -168,27 +169,39 @@ def test_fused_bn_relu_maxpool_matches_separate_passes(dev, N, C, H, W):
         bnm.weight.uniform_(0.5, 1.5)
         bnm.bias.normal_(0, 0.3)
     bnm.train()
-    xf = x0.float()
-    mean = xf.mean((0, 2, 3))
-    var = xf.var((0, 2, 3), unbiased=False)
-    rstd = torch.rsqrt(var + bnm.eps)
-    sb = torch.cat([bnm.weight.detach() * rstd, bnm.bias.detach() - mean * bnm.weight.detach() * rstd]).contiguous()
-    stats = dict(mean=mean.contiguous(), rstd=rstd.contiguous(), scale_bias=sb, momentum=0.1)
-    pool = MaxPool3x3s2()
+
+    def affine(x, gamma, beta):
+        mean = x.mean((0, 2, 3))
+        rstd = torch.rsqrt(x.var((0, 2, 3), unbiased=False) + bnm.eps)
+        return mean, rstd, gamma * rstd, beta - mean * gamma * rstd
+
+    mean, rstd, scale, bias = affine(x0.float(), bnm.weight.detach(), bnm.bias.detach())
+    stats = dict(mean=mean.contiguous(), rstd=rstd.contiguous(), scale_bias=torch.cat([scale, bias]).contiguous(), momentum=0.1)
 
     xa = x0.clone().requires_grad_()
-    ya = pool(bnm.apply_pre(xa, stats))
-    dy = torch.randn_like(ya)
-    ya.backward(dy)
-    ga, ba = bnm.weight.grad.clone(), bnm.bias.grad.clone()
-    bnm.weight.grad = bnm.bias.grad = None
-
-    xb = x0.clone().requires_grad_()
-    yb = BN.bn_relu_maxpool(bnm, xb, stats)
-    yb.backward(dy)
+    y = MaxPool3x3s2()(bnm.apply_pre(xa, stats))
+    dy = torch.randn_like(y)
+    y.backward(dy)
     torch.cuda.synchronize()
-    torch.testing.assert_close(yb.float(), ya.float(), rtol=0, atol=0)
-    torch.testing.assert_close(bnm.weight.grad, ga, rtol=2e-3, atol=2e-3 * float(ga.abs().max()))
-    torch.testing.assert_close(bnm.bias.grad, ba, rtol=2e-3, atol=2e-3 * float(ba.abs().max()))
-    d = (xb.grad.float() - xa.grad.float()).abs()
-    assert float(d.max()) <= 2e-2 * float(xa.grad.float().abs().max()) + 1e-6, float(d.max())
+
+    # the kernel rounds fmaf(x, scale, bias) to bf16.  In fp64 the product of a bf16 and an fp32 value is exact and the sum keeps
+    # 29 bits more than fp32, so t rounds to the same fp32 value, and its sign is the ReLU decision the kernel made
+    with torch.no_grad():
+        t = x0.double() * scale.double().view(1, -1, 1, 1) + bias.double().view(1, -1, 1, 1)
+        y1 = torch.relu(t).float().to(torch.bfloat16).float()
+        keep = (t > 0).float()
+    torch.testing.assert_close(y.float(), torch.nn.functional.max_pool2d(y1, 3, 2, 1), rtol=0, atol=0)
+
+    # backward: BatchNorm with batch statistics (mean and variance are functions of x) in fp32; the pooled values are the
+    # kernel's bf16 ones (straight-through), so that max_pool2d picks the same window maxima and routes dy to the same pixels
+    xr = x0.float().requires_grad_()
+    gr = bnm.weight.detach().clone().requires_grad_()
+    br = bnm.bias.detach().clone().requires_grad_()
+    _, _, sr, bir = affine(xr, gr, br)
+    lin = (xr * sr.view(1, -1, 1, 1) + bir.view(1, -1, 1, 1)) * keep
+    lin = lin + (y1 - lin).detach()
+    torch.nn.functional.max_pool2d(lin, 3, 2, 1).backward(dy.float())
+    torch.testing.assert_close(bnm.weight.grad, gr.grad, rtol=2e-3, atol=2e-3 * float(gr.grad.abs().max()))
+    torch.testing.assert_close(bnm.bias.grad, br.grad, rtol=2e-3, atol=2e-3 * float(br.grad.abs().max()))
+    d = (xa.grad.float() - xr.grad).abs()
+    assert float(d.max()) <= 2e-2 * float(xr.grad.abs().max()) + 1e-6, float(d.max())

@@ -49,15 +49,6 @@ class _ShadowConvFn(torch.autograd.Function):
         return dx, None, None, None, None, None, None
 
 
-def _bn_red_on() -> bool:
-    """V6B200_BN_RED=1: BatchNorm backward reduction in the data-gradient epilogue (csrc/igemm.cu EPI_RED).  Off by default:
-    measured 51.5 vs 50.5 ms per ResNet-50 round -- the x read and the arithmetic move into an epilogue that is already the
-    bottleneck of the memory-bound layers, and the dy re-read it saves was an L2 hit."""
-    import os
-
-    return os.environ.get("V6B200_BN_RED", "0") == "1"
-
-
 def _tc_mode() -> str:
     """V6B200_CONV = tc (default: the hand-written tcgen05 implicit-GEMM kernels, csrc/igemm.cu) | cudnn (library arm)."""
     import os
@@ -137,7 +128,7 @@ class _TcConvFn(torch.autograd.Function):
     ``weight.grad`` (the flat gradient buffer) -- no bf16 gradient tensor, no gradient sink entry."""
 
     @staticmethod
-    def forward(ctx, x, weight, w_bf16, stride, pad, bn, fork_in=None, fork_out=None, bnlink=None):
+    def forward(ctx, x, weight, w_bf16, stride, pad, bn, fork_in=None, fork_out=None):
         from ..ops import conv as C
 
         y = C.conv_fprop(x, w_bf16, stride, pad, bn=bn)
@@ -147,12 +138,6 @@ class _TcConvFn(torch.autograd.Function):
         ctx.fork_in, ctx.fork_out = fork_in, fork_out
         if fork_in is not None and stride == 1:
             fork_in.armed = True            # this node will fold the parked gradient into its data-gradient epilogue
-        # bnlink: x is the output of a BatchNorm whose COMPLETE output gradient this node's data-gradient kernel produces (sole
-        # consumer, or the other branch is absorbed through fork_in): that kernel then also does the BN's reduction pass
-        cout, cin, r, s = w_bf16.shape
-        ctx.bnlink = bnlink if (bnlink is not None and stride == 1 and fork_out is None and cin % 64 == 0 and cin <= 2048
-                                and C.dgrad_supported(cin, cout, r, s, stride, pad, x.shape[2], x.shape[3])
-                                and (fork_in is None or fork_in.armed)) else None
         return y
 
     @staticmethod
@@ -172,8 +157,7 @@ class _TcConvFn(torch.autograd.Function):
                 add, add_mask = ctx.fork_in.grad, ctx.fork_in.mask
                 ctx.fork_in.grad = ctx.fork_in.mask = None
             if C.dgrad_supported(cin, cout, r, s, stride, pad, x.shape[2], x.shape[3]):
-                red = ctx.bnlink.reduction_args() if (ctx.bnlink is not None and _bn_red_on()) else None
-                dx = C.conv_dgrad(dy, w_bf16, (x.shape[2], x.shape[3]), pad, stride=stride, add=add, add_mask=add_mask, bn_red=red)
+                dx = C.conv_dgrad(dy, w_bf16, (x.shape[2], x.shape[3]), pad, stride=stride, add=add, add_mask=add_mask)
                 add = None
             else:       # odd spatial sizes under stride 2: library kernel
                 dx = torch.ops.aten.convolution_backward(dy, x, w_bf16, None, (stride, stride), (pad, pad), (1, 1), False, (0, 0), 1,
@@ -195,10 +179,10 @@ class _TcConvFn(torch.autograd.Function):
                 _side.forked = True
             else:
                 C.conv_wgrad(dy, x, g, (r, s), stride, pad)
-            return dx, None, None, None, None, None, None, None, None
+            return dx, None, None, None, None, None, None, None
         dw = torch.zeros((cout, r, s, cin), device=x.device, dtype=torch.float32)
         C.conv_wgrad(dy, x, dw, (r, s), stride, pad)
-        return dx, dw.permute(0, 3, 1, 2), None, None, None, None, None, None, None
+        return dx, dw.permute(0, 3, 1, 2), None, None, None, None, None, None
 
 
 class ShadowConv2d(nn.Conv2d):
@@ -237,48 +221,21 @@ class ShadowConv2d(nn.Conv2d):
                                    self._offset)
 
 
-def _fuse_stats(conv: nn.Module) -> bool:
-    """BatchNorm statistics in the convolution epilogue only when the layer has at least ``V6B200_CONV_STATS_MIN_KB``
-    64-wide k-blocks (default 0 = always)."""
-    import os
-
-    min_kb = int(os.environ.get("V6B200_CONV_STATS_MIN_KB", "0"))
-    return conv.kernel_size[0] * conv.kernel_size[1] * conv.in_channels // 64 >= min_kb
-
-
-def _bn_with_fork(bn, y, residual, res_fork):
-    from ..ops.bn import _BNFn
-
-    mom = 0.1 if bn.momentum is None else bn.momentum
-    return _BNFn.apply(y, residual, bn.weight, bn.bias, bn.running_mean, bn.running_var, bn.num_batches_tracked, bn.eps, mom,
-                       bn.relu, None, res_fork)
-
-
 def conv_bn(conv: nn.Module, bn: nn.Module, x: torch.Tensor, residual: Optional[torch.Tensor] = None,
-            fork_in: Optional[GradFork] = None, fork_out: Optional[GradFork] = None, res_fork: Optional[GradFork] = None,
-            absorb: bool = False) -> torch.Tensor:
+            fork_in: Optional[GradFork] = None, fork_out: Optional[GradFork] = None, res_fork: Optional[GradFork] = None) -> torch.Tensor:
     """``bn(conv(x), residual)``.  On the tcgen05 path the BatchNorm batch statistics come out of the convolution's
     epilogue (one launch less and one full read of the activation less per layer); everywhere else the two modules are
     simply composed.  ``fork_in`` / ``fork_out`` / ``res_fork``: see :class:`GradFork` (``fork_in``: this convolution's
     data gradient absorbs the parked gradient; ``fork_out``: this convolution parks its data gradient; ``res_fork``: the
-    BatchNorm parks the gradient of its residual input).  ``absorb``: ``x`` is a BatchNorm output that only this convolution
-    consumes (or ``fork_in`` brings in the other branch): its data-gradient kernel also does that BatchNorm's backward
-    reduction pass (ops/bn.py::BNLink)."""
-    from ..ops.bn import FusedBatchNormAct, bn_link_of
-
-    link = bn_link_of(x) if (absorb or fork_in is not None) and x.is_cuda and fork_out is None else None
+    BatchNorm parks the gradient of its residual input)."""
+    from ..ops.bn import FusedBatchNormAct
 
     if (isinstance(conv, ShadowConv2d) and isinstance(bn, FusedBatchNormAct) and bn.training and torch.is_grad_enabled()
             and conv.w_bf16 is not None and conv.weight.requires_grad and x.is_cuda):
         if x.dtype != torch.bfloat16:
             x = x.to(torch.bfloat16)
         if conv.tc_supported(x) and (residual is None or residual.is_contiguous(memory_format=torch.channels_last)):
-            if not _fuse_stats(conv):
-                # short reduction dimension: the convolution is bound by its epilogue, where the statistics are not free;
-                # the separate statistics pass reads an output that is still (partly) in L2
-                y = _TcConvFn.apply(x, conv.weight, conv.w_bf16, conv.stride[0], conv.padding[0], None, fork_in, fork_out, link)
-                return _bn_with_fork(bn, y, residual, res_fork)
             stats = bn.stats_buffers(x.device)
-            y = _TcConvFn.apply(x, conv.weight, conv.w_bf16, conv.stride[0], conv.padding[0], stats, fork_in, fork_out, link)
+            y = _TcConvFn.apply(x, conv.weight, conv.w_bf16, conv.stride[0], conv.padding[0], stats, fork_in, fork_out)
             return bn.apply_pre(y, stats, residual, res_fork=res_fork)
     return bn(conv(x), residual=residual) if residual is not None else bn(conv(x))

@@ -65,13 +65,11 @@ class Bottleneck(nn.Module):
         # conv1's data-gradient kernel instead of being added by a separate pass (GradFork; only armed on the tcgen05 path)
         fork = GradFork() if (self.training and torch.is_grad_enabled() and x.requires_grad) else None
         out = conv_bn(self.conv1, self.bn1, x, fork_in=fork)       # conv (+ BN statistics in its epilogue) -> BN apply + ReLU
-        # absorb: conv2 / conv3 are the only consumers of bn1 / bn2's outputs -> their data-gradient kernels also do the
-        # reduction pass of those BatchNorms' backward (conv1 does it for the previous block's bn3 through the fork)
-        out = conv_bn(self.conv2, self.bn2, out, absorb=True)
+        out = conv_bn(self.conv2, self.bn2, out)
         if self.downsample is None:
-            return conv_bn(self.conv3, self.bn3, out, residual=x, res_fork=fork, absorb=True)     # BN + residual add + ReLU in one pass
+            return conv_bn(self.conv3, self.bn3, out, residual=x, res_fork=fork)     # BN + residual add + ReLU in one pass
         idt = conv_bn(self.downsample[0], self.downsample[1], x, fork_out=fork)
-        return conv_bn(self.conv3, self.bn3, out, residual=idt, absorb=True)
+        return conv_bn(self.conv3, self.bn3, out, residual=idt)
 
 
 class ResNet(nn.Module):
@@ -108,10 +106,9 @@ class ResNet(nn.Module):
         layers += [Bottleneck(self.inplanes, planes, fused_bn=self.fused_bn) for _ in range(1, blocks)]
         return nn.Sequential(*layers)
 
-    def _stem(self, x: torch.Tensor, with_pool: bool = False):
+    def _stem(self, x: torch.Tensor) -> torch.Tensor:
         """conv1 + bn1(+ReLU).  uint8 NCHW images are normalised on the GPU (the host only ships raw bytes);
-        on the fused path the stem runs as a space-to-depth 4x4 convolution (ops/pool.py::stem_s2d).  ``with_pool``: the
-        caller applies ``self.maxpool`` next -- when the fused pass exists the result is ``(pooled tensor, True)``."""
+        on the fused path the stem runs as a space-to-depth 4x4 convolution (ops/pool.py::stem_s2d)."""
         if x.dtype != torch.uint8:
             return self.bn1(self.conv1(x.contiguous(memory_format=torch.channels_last)))
         bf16_stem = torch.is_autocast_enabled() or getattr(self.conv1, "w_bf16", None) is not None
@@ -119,16 +116,9 @@ class ResNet(nn.Module):
             from ..ops import pool
 
             if pool.stem_s2d_supported(x, self.conv1):
-                from .conv import _fuse_stats
-
-                if (self.training and pool.stem_stats_fused(self.conv1) and hasattr(self.bn1, "stats_buffers") and _fuse_stats(self.layer1[0].conv3)):
+                if self.training and pool.stem_stats_fused(self.conv1) and hasattr(self.bn1, "stats_buffers"):
                     stats = self.bn1.stats_buffers(x.device)        # batch statistics out of the convolution's epilogue
                     y = pool.stem_s2d(x, self.conv1, _MEAN, _STD, bn=stats)
-                    if with_pool:
-                        from ..ops.bn import bn_pool_fusable, bn_relu_maxpool
-
-                        if bn_pool_fusable(self.bn1, self.maxpool, y):
-                            return bn_relu_maxpool(self.bn1, y, stats), True      # BN apply + ReLU + max-pool as one pass
                     return self.bn1.apply_pre(y, stats)
                 return self.bn1(pool.stem_s2d(x, self.conv1, _MEAN, _STD))
             if x.is_contiguous() and (x.shape[2] * x.shape[3]) % 4 == 0:
@@ -142,8 +132,7 @@ class ResNet(nn.Module):
         return self.bn1(self.conv1(x))
 
     def forward(self, x):
-        x = self._stem(x, with_pool=True)
-        x = x[0] if isinstance(x, tuple) else self.maxpool(x)        # (pooled, True): the stem did BN + ReLU + max-pool in one pass
+        x = self.maxpool(self._stem(x))
         x = self.layer4(self.layer3(self.layer2(self.layer1(x))))
         return self.fc(torch.flatten(self.avgpool(x), 1))
 

@@ -40,40 +40,6 @@ def _fast_path(x: torch.Tensor) -> bool:
     return C % 8 == 0 and 1 <= cg <= 256 and (cg & (cg - 1)) == 0 and x.is_contiguous(memory_format=torch.channels_last)
 
 
-class BNLink:
-    """Hand-over between a BatchNorm node and the convolution that consumes its output: in the backward pass that
-    convolution's data-gradient kernel produces the BN's output gradient and -- when it is the only consumer, or absorbs the
-    other branch (models/conv.py::GradFork) -- can do the BN's reduction pass (sum g, sum g.xhat -> dgamma, dbeta, the
-    coefficients of dx) in its epilogue (ops/conv.py ``bn_red=``).  ``reduced`` then tells the BN node to run only its
-    element-wise half."""
-
-    __slots__ = ("x", "mask", "mean", "rstd", "gamma", "params", "relu", "reduced", "coef", "dgamma", "dbeta", "direct")
-
-    def __init__(self, x, mask, mean, rstd, gamma, params, relu):
-        self.x, self.mask, self.mean, self.rstd, self.gamma, self.params, self.relu = x, mask, mean, rstd, gamma, params, relu
-        self.reduced, self.coef, self.dgamma, self.dbeta, self.direct = False, None, None, None, False
-
-    def reduction_args(self) -> dict:
-        """Arguments for ``conv_dgrad(bn_red=...)``; marks the reduction as done."""
-        pg, pb = self.params
-        self.direct = all(p.grad is not None and p.grad.dtype == torch.float32 and p.grad.is_contiguous() for p in (pg, pb))
-        C = self.gamma.numel()
-        self.dgamma = pg.grad if self.direct else torch.empty(C, device=self.x.device, dtype=torch.float32)
-        self.dbeta = pb.grad if self.direct else torch.empty(C, device=self.x.device, dtype=torch.float32)
-        self.coef = torch.empty(3 * C, device=self.x.device, dtype=torch.float32)
-        self.reduced = True
-        return dict(x=self.x, mask=self.mask if self.relu else None, mean=self.mean, rstd=self.rstd, gamma=self.gamma,
-                    dgamma=self.dgamma, dbeta=self.dbeta, coef=self.coef, accumulate=self.direct)
-
-
-def bn_link_of(t: torch.Tensor):
-    """The :class:`BNLink` of the BatchNorm node that produced ``t`` (None for any other tensor)."""
-    link = getattr(t, "_v6_bnlink", None)
-    if link is None and t.grad_fn is not None:
-        link = getattr(t.grad_fn, "link", None)
-    return link if isinstance(link, BNLink) else None
-
-
 class _BNFn(torch.autograd.Function):
     @staticmethod
     def forward(ctx, x, residual, gamma, beta, running_mean, running_var, num_batches_tracked, eps, momentum, relu, pre=None,
@@ -106,8 +72,6 @@ class _BNFn(torch.autograd.Function):
         ctx.relu, ctx.has_res, ctx.R, ctx.C = relu, residual is not None, R, C
         ctx.params = (gamma, beta)
         ctx.res_fork = res_fork             # models/conv.py::GradFork: park the residual gradient for the block's first conv
-        ctx.link = BNLink(x, mask, mean, rstd, gamma, (gamma, beta), relu)
-        y._v6_bnlink = ctx.link             # read by the consuming convolution (models/conv.py::_TcConvFn)
         return y
 
     @staticmethod
@@ -126,82 +90,16 @@ class _BNFn(torch.autograd.Function):
         direct = all(p.grad is not None and p.grad.dtype == torch.float32 and p.grad.is_contiguous() for p in (pg, pb))
         dgamma = pg.grad if direct else torch.empty_like(gamma)
         dbeta = pb.grad if direct else torch.empty_like(gamma)
-        link = ctx.link
-        if link is not None and link.reduced:
-            # the data-gradient kernel that produced dy already did the reduction pass (dgamma, dbeta, coefficients)
-            direct, dgamma, dbeta = link.direct, link.dgamma, link.dbeta
-            count(1)
-            native().bn_bwd_apply(dy.data_ptr(), 0 if mask is None else mask.data_ptr(), x.data_ptr(), link.coef.data_ptr(), dx.data_ptr(),
-                                  0 if dres is None else dres.data_ptr(), ctx.R, ctx.C, ctx.relu, stream_ptr())
-        else:
-            part, coef = _get_scratch(x.device, ctx.C)
-            count(2)                                             # reduce(+finalize) + apply
-            native().bn_bwd(dy.data_ptr(), 0 if mask is None else mask.data_ptr(), x.data_ptr(), gamma.data_ptr(), mean.data_ptr(),
-                            rstd.data_ptr(), dx.data_ptr(), 0 if dres is None else dres.data_ptr(), dgamma.data_ptr(),
-                            dbeta.data_ptr(), coef.data_ptr(), part.data_ptr(), ctx.R, ctx.C, ctx.relu, direct, stream_ptr())
+        part, coef = _get_scratch(x.device, ctx.C)
+        count(2)                                                 # reduce(+finalize) + apply
+        native().bn_bwd(dy.data_ptr(), 0 if mask is None else mask.data_ptr(), x.data_ptr(), gamma.data_ptr(), mean.data_ptr(),
+                        rstd.data_ptr(), dx.data_ptr(), 0 if dres is None else dres.data_ptr(), dgamma.data_ptr(),
+                        dbeta.data_ptr(), coef.data_ptr(), part.data_ptr(), ctx.R, ctx.C, ctx.relu, direct, stream_ptr())
         if park:
             ctx.res_fork.grad, ctx.res_fork.mask = dy, (mask if ctx.relu else None)
         if direct:
             return dx, dres, None, None, None, None, None, None, None, None, None, None
         return dx, dres, dgamma, dbeta, None, None, None, None, None, None, None, None
-
-
-class _BNPoolFn(torch.autograd.Function):
-    """``maxpool3x3s2p1(relu(bn(x)))`` of the ResNet stem as one pass in each direction (csrc/bn.cu: bn_relu_maxpool_fwd_kernel,
-    bn_pool_bwd_*): the 112 x 112 BatchNorm output, its ReLU mask and the 112 x 112 gradient the max-pool backward would
-    write never exist.  The batch statistics come from the stem convolution's epilogue (``pre``)."""
-
-    @staticmethod
-    def forward(ctx, x, gamma, beta, pre):
-        mean, rstd, scale_bias = pre
-        n, c, h, w = x.shape
-        ho, wo = (h - 1) // 2 + 1, (w - 1) // 2 + 1
-        p = torch.empty((n, c, ho, wo), device=x.device, dtype=torch.bfloat16, memory_format=torch.channels_last)
-        idx = torch.empty((n, ho, wo, c), device=x.device, dtype=torch.uint8)
-        count(1)
-        native().bn_pool_fwd(x.data_ptr(), scale_bias.data_ptr(), scale_bias.data_ptr() + 4 * c, p.data_ptr(), idx.data_ptr(), n, h, w, c,
-                             stream_ptr())
-        ctx.save_for_backward(x, idx, gamma, mean, rstd, scale_bias)
-        ctx.params = (gamma, beta)
-        return p
-
-    @staticmethod
-    def backward(ctx, dp):
-        x, idx, gamma, mean, rstd, scale_bias = ctx.saved_tensors
-        if not dp.is_contiguous(memory_format=torch.channels_last):
-            dp = dp.contiguous(memory_format=torch.channels_last)
-        n, c, h, w = x.shape
-        dx = torch.empty_like(x)
-        pg, pb = ctx.params
-        direct = all(p.grad is not None and p.grad.dtype == torch.float32 and p.grad.is_contiguous() for p in (pg, pb))
-        dgamma = pg.grad if direct else torch.empty_like(gamma)
-        dbeta = pb.grad if direct else torch.empty_like(gamma)
-        part, _ = _get_scratch(x.device, c)
-        coef = torch.empty(3 * c, device=x.device, dtype=torch.float32)
-        count(2)
-        native().bn_pool_bwd(dp.data_ptr(), idx.data_ptr(), x.data_ptr(), scale_bias.data_ptr(), scale_bias.data_ptr() + 4 * c,
-                             gamma.data_ptr(), mean.data_ptr(), rstd.data_ptr(), dx.data_ptr(), dgamma.data_ptr(), dbeta.data_ptr(),
-                             coef.data_ptr(), part.data_ptr(), n, h, w, c, direct, stream_ptr())
-        if direct:
-            return dx, None, None, None
-        return dx, dgamma, dbeta, None
-
-
-def bn_relu_maxpool(bn: "FusedBatchNormAct", x: torch.Tensor, stats: dict) -> torch.Tensor:
-    """Training-time ``maxpool(relu(bn(x)))`` with the batch statistics in ``stats`` (filled by the producing convolution)."""
-    return _BNPoolFn.apply(x, bn.weight, bn.bias, (stats["mean"], stats["rstd"], stats["scale_bias"]))
-
-
-def bn_pool_fusable(bn, pool, x: torch.Tensor) -> bool:
-    import os
-
-    from .pool import MaxPool3x3s2
-
-    # opt-in (V6B200_STEM_POOL=fused): correct (tests/test_gpu_resnet_ops.py) but measured 51.1 vs 50.4 ms per ResNet-50 round --
-    # the per-pixel gather of the pooled gradient in BOTH backward passes and the 9-tap affine + ReLU in the forward cost more
-    # than the 2 x 103 MB per step they avoid
-    return (os.environ.get("V6B200_STEM_POOL", "separate") == "fused" and isinstance(bn, FusedBatchNormAct) and bn.relu and bn.training
-            and isinstance(pool, MaxPool3x3s2) and x.is_cuda and torch.is_grad_enabled() and bn.num_features % 64 == 0)
 
 
 class FusedBatchNormAct(nn.BatchNorm2d):

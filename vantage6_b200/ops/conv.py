@@ -90,8 +90,7 @@ def conv_fprop(x: torch.Tensor, w: torch.Tensor, stride: int = 1, pad: int = 0, 
 
 
 def conv_dgrad(dy: torch.Tensor, w: torch.Tensor, in_hw: Tuple[int, int], pad: int = 0, force_im2col: bool = False,
-               stride: int = 1, add: Optional[torch.Tensor] = None, add_mask: Optional[torch.Tensor] = None,
-               bn_red: Optional[dict] = None) -> torch.Tensor:
+               stride: int = 1, add: Optional[torch.Tensor] = None, add_mask: Optional[torch.Tensor] = None) -> torch.Tensor:
     """Data gradient of a convolution: ``dy`` [N, Cout, P, Q] -> dx [N, Cin, H, W] (channels_last bf16).  stride 2 (3x3 /
     pad 1 and 1x1 / pad 0, even H, W): one launch that walks the 4 output-pixel parity classes, each a stride-1 implicit
     GEMM over dY with the sub-filter that reaches it."""
@@ -105,19 +104,9 @@ def conv_dgrad(dy: torch.Tensor, w: torch.Tensor, in_hw: Tuple[int, int], pad: i
         assert add.shape == dx.shape and add.dtype == torch.bfloat16 and _is_cl(add) and stride == 1
         # add_mask: 1 bit / element ([pixels, C/8] bytes, ops/bn.py): the branch gradient is ``add`` where the bit is set, else 0
         assert add_mask is None or (add_mask.dtype == torch.uint8 and add_mask.numel() * 8 == add.numel())
-    red = [0] * 8 + [False, 0]
-    if bn_red is not None:
-        # the reduction pass of the BatchNorm backward that consumes dx, in this kernel's epilogue (csrc/igemm.cu EPI_RED):
-        # bn_red = dict(x, mask, mean, rstd, gamma, dgamma, dbeta, coef, accumulate) of that BatchNorm; dx must be the COMPLETE
-        # gradient of the BN output (``add`` included)
-        assert stride == 1 and cin % 64 == 0 and bn_red["x"].shape == dx.shape and _is_cl(bn_red["x"])
-        m = bn_red.get("mask")
-        red = [bn_red["x"].data_ptr(), 0 if m is None else m.data_ptr(), bn_red["mean"].data_ptr(), bn_red["rstd"].data_ptr(),
-               bn_red["gamma"].data_ptr(), bn_red["dgamma"].data_ptr(), bn_red["dbeta"].data_ptr(), bn_red["coef"].data_ptr(),
-               bool(bn_red["accumulate"]), igemm_scratch(dy.device).data_ptr()]
     count(1)
     native().conv_dgrad(dy.data_ptr(), w.data_ptr(), dx.data_ptr(), n, h, wd, cin, cout, r, s, stride, pad, force_im2col, stream_ptr(),
-                        0 if add is None else add.data_ptr(), 0 if (add is None or add_mask is None) else add_mask.data_ptr(), *red)
+                        0 if add is None else add.data_ptr(), 0 if (add is None or add_mask is None) else add_mask.data_ptr())
     return dx
 
 
@@ -212,7 +201,7 @@ def linear_dgrad(dy: torch.Tensor, w: torch.Tensor) -> torch.Tensor:
     assert n == n2
     dx = torch.empty((m, k), device=dy.device, dtype=torch.bfloat16)
     count(1)
-    native().conv_dgrad(dy.data_ptr(), w.data_ptr(), dx.data_ptr(), 1, 1, m, k, n, 1, 1, 1, 0, False, stream_ptr(), 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, False, 0)
+    native().conv_dgrad(dy.data_ptr(), w.data_ptr(), dx.data_ptr(), 1, 1, m, k, n, 1, 1, 1, 0, False, stream_ptr(), 0, 0)
     return dx
 
 

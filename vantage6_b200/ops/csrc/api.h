@@ -154,12 +154,6 @@ int v6_ce_fwd(const void* logits, const long long* labels, float* lse, float* lo
               cudaStream_t s);
 int v6_ce_bwd(void* logits, const long long* labels, const float* lse, const float* scale_ptr, int T, int V, int V_alloc, long long ld,
               long long ignore_index, cudaStream_t s);
-int v6_bn_pool_fwd(const void* x, const float* scale, const float* bias, void* p, void* idx, int N, int H, int W, int C, cudaStream_t s);
-int v6_bn_pool_bwd(const void* dp, const void* idx, const void* x, const float* scale, const float* bias, const float* gamma, const float* mean,
-                   const float* rstd, void* dx, float* dgamma, float* dbeta, float* coef, float* scratch, int N, int H, int W, int C,
-                   int accumulate, cudaStream_t s);
-int v6_bn_bwd_apply(const void* dy, const void* relu_mask, const void* x, const float* coef, void* dx, void* dres, long long R, int C,
-                    int relu, cudaStream_t s);
 int v6_bn_bwd(const void* dy, const void* relu_mask, const void* x, const float* gamma, const float* mean, const float* rstd, void* dx,
               void* dres, float* dgamma, float* dbeta, float* coef, float* scratch, long long R, int C, int relu,
               int accumulate, cudaStream_t s);
@@ -202,9 +196,7 @@ int v6_conv_fprop(const void* x, const void* w, void* y, const float* bias, int 
                   float eps, float momentum, int force_im2col, long long pitch_w, long long pitch_h, long long pitch_n,
                   cudaStream_t stream);
 int v6_conv_dgrad(const void* dy, const void* w, void* dx, int N, int H, int W, int Cin, int Cout, int R, int S, int stride, int pad,
-                  int force_im2col, const void* add_src, const void* add_mask, const void* red_x, const void* red_mask,
-                  const float* red_mean, const float* red_rstd, const float* red_gamma, float* red_dgamma, float* red_dbeta, float* red_coef,
-                  int red_accumulate, float* scratch, cudaStream_t stream);
+                  int force_im2col, const void* add_src, const void* add_mask, cudaStream_t stream);
 int v6_conv_wgrad(const void* dy, const void* x, float* dw, int N, int H, int W, int Cin, int Cout, int R, int S, int stride, int pad,
                   float scale, int splits, int force_im2col, long long pitch_w, long long pitch_h, long long pitch_n,
                   float* ws, long long ws_floats, cudaStream_t stream);

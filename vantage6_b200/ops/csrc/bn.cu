@@ -108,25 +108,19 @@ __global__ void __launch_bounds__(THREADS, 4) bn_stats_kernel(const __nv_bfloat1
 
 // Element-wise passes: U rows per thread are requested (raw 16 B vectors, kept packed until used) before the first one
 // is consumed, and the grid is exactly one wave of resident CTAs (apply_grid) -- HBM3e wants >= ~64 KB of loads in flight
-// per SM and a grid-stride loop has no tail.  SMEM_COEF keeps the per-channel coefficients in shared memory instead of
-// 16-24 registers so that 4 CTAs/SM stay resident with U = 4.
-template <bool RELU, bool RES, int U, int MINB, bool SMEM_COEF>
+// per SM and a grid-stride loop has no tail.  Launched with U = 2 at 3 CTAs/SM, coefficients in registers:
+// 2.52 ms of these passes per ResNet-50 step on a B200, vs 2.93 ms with U = 4 at 4 CTAs/SM (coefficients in shared memory) and 2.51 ms with U = 4 at 2 CTAs/SM (profiles/bn_bench_r2f.jsonl).
+template <bool RELU, bool RES, int U, int MINB>
 __global__ void __launch_bounds__(THREADS, MINB) bn_apply_kernel(const __nv_bfloat16* __restrict__ x, const __nv_bfloat16* __restrict__ res,
                                                                  const float* __restrict__ scale, const float* __restrict__ bias,
                                                                  __nv_bfloat16* __restrict__ y, unsigned char* __restrict__ mask,
                                                                  long long R, int C) {
-    extern __shared__ float s_coef[];                           // SMEM_COEF: scale[C] | bias[C]
     const int CG = C >> 3, RL = THREADS / CG;
     const int cg = threadIdx.x % CG, rl = threadIdx.x / CG;
     pdl_wait();                                                 // scale / bias come from the stats kernel
     float sc[8], bi[8];
-    if (SMEM_COEF) {
-        for (int i = threadIdx.x; i < C; i += THREADS) { s_coef[i] = scale[i]; s_coef[C + i] = bias[i]; }
-        __syncthreads();
-    } else {
-        loadf8(scale + cg * 8, sc);
-        loadf8(bias + cg * 8, bi);
-    }
+    loadf8(scale + cg * 8, sc);
+    loadf8(bias + cg * 8, bi);
     const long long G = (long long)gridDim.x * RL;
     for (long long r0 = (long long)blockIdx.x * RL + rl; r0 < R; r0 += U * G) {
         uint4 xr[U], qr[U];
@@ -145,7 +139,6 @@ __global__ void __launch_bounds__(THREADS, MINB) bn_apply_kernel(const __nv_bflo
                 float v[8], q[8];
                 unpack8(xr[u], v);
                 if (RES) unpack8(qr[u], q);
-                if (SMEM_COEF) { loadf8(s_coef + cg * 8, sc); loadf8(s_coef + C + cg * 8, bi); }
                 unsigned bits = 0;
 #pragma unroll
                 for (int k = 0; k < 8; ++k) {
@@ -234,24 +227,18 @@ __global__ void __launch_bounds__(THREADS, 3) bn_bwd_reduce_kernel(const __nv_bf
     }
 }
 
-template <bool RELU, bool RES, int U, int MINB, bool SMEM_COEF>
+template <bool RELU, bool RES, int U, int MINB>
 __global__ void __launch_bounds__(THREADS, MINB) bn_bwd_apply_kernel(const __nv_bfloat16* __restrict__ dy, const unsigned char* __restrict__ mask,
                                                                      const __nv_bfloat16* __restrict__ x, const float* __restrict__ coef,
                                                                      __nv_bfloat16* __restrict__ dx, __nv_bfloat16* __restrict__ dres,
                                                                      long long R, int C) {
-    extern __shared__ float s_coef[];                           // SMEM_COEF: c0[C] | c1[C] | c2[C]
     const int CG = C >> 3, RL = THREADS / CG;
     const int cg = threadIdx.x % CG, rl = threadIdx.x / CG;
     pdl_wait();                                                 // coefficients come from the reduce kernel
     float c0[8], c1[8], c2[8];
-    if (SMEM_COEF) {
-        for (int i = threadIdx.x; i < 3 * C; i += THREADS) s_coef[i] = coef[i];
-        __syncthreads();
-    } else {
-        loadf8(coef + cg * 8, c0);
-        loadf8(coef + C + cg * 8, c1);
-        loadf8(coef + 2 * C + cg * 8, c2);
-    }
+    loadf8(coef + cg * 8, c0);
+    loadf8(coef + C + cg * 8, c1);
+    loadf8(coef + 2 * C + cg * 8, c2);
     const long long G = (long long)gridDim.x * RL;
     for (long long r0 = (long long)blockIdx.x * RL + rl; r0 < R; r0 += U * G) {
         uint4 gr[U], xr[U];
@@ -273,7 +260,6 @@ __global__ void __launch_bounds__(THREADS, MINB) bn_bwd_apply_kernel(const __nv_
                 float g[8], xv[8], o[8];
                 unpack8(gr[u], g);
                 unpack8(xr[u], xv);
-                if (SMEM_COEF) { loadf8(s_coef + cg * 8, c0); loadf8(s_coef + C + cg * 8, c1); loadf8(s_coef + 2 * C + cg * 8, c2); }
 #pragma unroll
                 for (int k = 0; k < 8; ++k) {
                     if (RELU && !((mb[u] >> k) & 1u)) g[k] = 0.f;
@@ -286,157 +272,6 @@ __global__ void __launch_bounds__(THREADS, MINB) bn_bwd_apply_kernel(const __nv_
     }
 }
 
-// ---------------------------------------------------------------------------------- stem: BN apply + ReLU + max-pool as one pass
-// y1 = relu(x * scale + bias) at 112 x 112 is only ever consumed by the 3x3 / s2 / p1 max-pool: the forward below reads the raw
-// convolution output and writes the pooled tensor + arg-max bytes (y1 and its ReLU mask never exist: 2 x 103 MB less per step at
-// batch 64); the backward gathers the pooled gradient on the fly (<= 4 windows per pixel), recomputes relu' from x, and runs
-// the usual reduce / apply pair -- the full-resolution gradient tensor that maxpool_bwd wrote and both BN passes re-read
-// never exists either.
-V6_DEVINL void pooled_grad(const __nv_bfloat16* __restrict__ dp, const unsigned char* __restrict__ idx, int n, int h, int w, int cg,
-                           int C, int Ho, int Wo, float (&acc)[8]) {
-#pragma unroll
-    for (int k = 0; k < 8; ++k) acc[k] = 0.f;
-    const int ho_lo = h >> 1, ho_hi = (h + 1) >> 1, wo_lo = w >> 1, wo_hi = (w + 1) >> 1;
-#pragma unroll
-    for (int a = 0; a < 2; ++a) {
-        const int ho = a ? ho_hi : ho_lo;
-        if ((a && ho_hi == ho_lo) || ho >= Ho) continue;
-        const int dh = h - (2 * ho - 1);
-#pragma unroll
-        for (int b = 0; b < 2; ++b) {
-            const int wo = b ? wo_hi : wo_lo;
-            if ((b && wo_hi == wo_lo) || wo >= Wo) continue;
-            const unsigned me = (unsigned)(dh * 3 + (w - (2 * wo - 1)));
-            const size_t o = ((size_t)(n * Ho + ho) * Wo + wo) * C + cg * 8;
-            const uint2 am = __ldg(reinterpret_cast<const uint2*>(idx + o));
-            float gv[8];
-            unpack8(ldg_nc_v4(dp + o), gv);
-#pragma unroll
-            for (int k = 0; k < 8; ++k) {
-                const unsigned ak = ((k < 4 ? am.x : am.y) >> (8 * (k & 3))) & 0xffu;
-                if (ak == me) acc[k] += gv[k];
-            }
-        }
-    }
-}
-
-// one thread = 8 channels of one pooled pixel
-__global__ void __launch_bounds__(THREADS) bn_relu_maxpool_fwd_kernel(const __nv_bfloat16* __restrict__ x, const float* __restrict__ scale,
-                                                                      const float* __restrict__ bias, __nv_bfloat16* __restrict__ p,
-                                                                      unsigned char* __restrict__ idx, int N, int H, int W, int C, int Ho, int Wo) {
-    const int CG = C >> 3;
-    const int total = N * Ho * Wo * CG;
-    pdl_wait();
-    for (int t = blockIdx.x * blockDim.x + threadIdx.x; t < total; t += gridDim.x * blockDim.x) {
-        const int cg = t % CG;
-        int q = t / CG;
-        const int wo = q % Wo; q /= Wo;
-        const int ho = q % Ho;
-        const int n = q / Ho;
-        float sc[8], bi[8];
-        loadf8(scale + cg * 8, sc);
-        loadf8(bias + cg * 8, bi);
-        const int h0 = 2 * ho - 1, w0 = 2 * wo - 1;
-        uint4 raw[9];
-#pragma unroll
-        for (int j = 0; j < 9; ++j) {
-            const int h = h0 + j / 3, w = w0 + j % 3;
-            if (h >= 0 && h < H && w >= 0 && w < W) raw[j] = ldg_nc_v4(x + ((size_t)(n * H + h) * W + w) * C + cg * 8);
-        }
-        float best[8];
-        unsigned arg[8];
-#pragma unroll
-        for (int k = 0; k < 8; ++k) { best[k] = -INFINITY; arg[k] = 0; }
-#pragma unroll
-        for (int j = 0; j < 9; ++j) {
-            const int h = h0 + j / 3, w = w0 + j % 3;
-            if (h >= 0 && h < H && w >= 0 && w < W) {
-                float v[8];
-                unpack8(raw[j], v);
-#pragma unroll
-                for (int k = 0; k < 8; ++k) {
-                    // the value the separate passes would have stored: relu(affine) rounded to bf16; first maximum in scan order
-                    const float yv = __bfloat162float(__float2bfloat16_rn(fmaxf(fmaf(v[k], sc[k], bi[k]), 0.f)));
-                    if (yv > best[k]) { best[k] = yv; arg[k] = j; }
-                }
-            }
-        }
-        const size_t o = ((size_t)(n * Ho + ho) * Wo + wo) * C + cg * 8;
-        store8(p + o, best);
-        *reinterpret_cast<uint2*>(idx + o) = make_uint2(arg[0] | (arg[1] << 8) | (arg[2] << 16) | (arg[3] << 24),
-                                                         arg[4] | (arg[5] << 8) | (arg[6] << 16) | (arg[7] << 24));
-    }
-}
-
-// reduce + finalize of the BN backward with g = pooled gradient . relu'(x * scale + bias)
-__global__ void __launch_bounds__(THREADS, 3) bn_pool_bwd_reduce_kernel(const __nv_bfloat16* __restrict__ dp, const unsigned char* __restrict__ idx,
-                                       const __nv_bfloat16* __restrict__ x, const float* __restrict__ scale, const float* __restrict__ bias,
-                                       const float* __restrict__ gamma, const float* __restrict__ mean, const float* __restrict__ rstd, Red rd,
-                                       float* __restrict__ dgamma, float* __restrict__ dbeta, float* __restrict__ coef,
-                                       int N, int H, int W, int C, int Ho, int Wo, int accumulate) {
-    __shared__ float tot[128];
-    const int SW = 64, CGS = 8, RL = THREADS / CGS;
-    const int cgl = threadIdx.x % CGS, rl = threadIdx.x / CGS;
-    const int cg = blockIdx.y * CGS + cgl;                    // channel group of the whole tensor
-    const size_t c0 = (size_t)cg * 8;
-    pdl_wait();
-    float mu[8], rs[8], sc[8], bi[8], sg[8], sgx[8];
-    loadf8(mean + c0, mu); loadf8(rstd + c0, rs); loadf8(scale + c0, sc); loadf8(bias + c0, bi);
-#pragma unroll
-    for (int k = 0; k < 8; ++k) { sg[k] = 0.f; sgx[k] = 0.f; }
-    const int R = N * H * W, G = gridDim.x * RL;
-    for (int r = blockIdx.x * RL + rl; r < R; r += G) {
-        const int w = r % W, q = r / W, h = q % H, n = q / H;
-        float xv[8], g[8];
-        unpack8(ldg_nc_v4(x + (size_t)r * C + c0), xv);
-        pooled_grad(dp, idx, n, h, w, cg, C, Ho, Wo, g);
-#pragma unroll
-        for (int k = 0; k < 8; ++k) {
-            const float gg = fmaf(xv[k], sc[k], bi[k]) > 0.f ? g[k] : 0.f;
-            sg[k] += gg;
-            sgx[k] = fmaf(gg, (xv[k] - mu[k]) * rs[k], sgx[k]);
-        }
-    }
-    pdl_launch_dependents();
-    if (!slice_reduce(sg, sgx, rd, SW, tot)) return;
-    if (threadIdx.x < SW) {
-        const int c = blockIdx.y * SW + threadIdx.x;
-        const float tg = tot[threadIdx.x], tgx = tot[SW + threadIdx.x];
-        dgamma[c] = accumulate ? dgamma[c] + tgx : tgx;
-        dbeta[c] = accumulate ? dbeta[c] + tg : tg;
-        const float invR = 1.f / (float)R;
-        const float k0 = gamma[c] * rstd[c];
-        const float k1 = -k0 * rstd[c] * tgx * invR;
-        coef[c] = k0;
-        coef[C + c] = k1;
-        coef[2 * C + c] = -k0 * tg * invR - k1 * mean[c];
-    }
-}
-
-__global__ void __launch_bounds__(THREADS, 3) bn_pool_bwd_apply_kernel(const __nv_bfloat16* __restrict__ dp, const unsigned char* __restrict__ idx,
-                                      const __nv_bfloat16* __restrict__ x, const float* __restrict__ scale, const float* __restrict__ bias,
-                                      const float* __restrict__ coef, __nv_bfloat16* __restrict__ dx, int N, int H, int W, int C, int Ho, int Wo) {
-    const int CG = C >> 3, RL = THREADS / CG;
-    const int cg = threadIdx.x % CG, rl = threadIdx.x / CG;
-    pdl_wait();
-    float c0[8], c1[8], c2[8], sc[8], bi[8];
-    loadf8(coef + cg * 8, c0); loadf8(coef + C + cg * 8, c1); loadf8(coef + 2 * C + cg * 8, c2);
-    loadf8(scale + cg * 8, sc); loadf8(bias + cg * 8, bi);
-    const int R = N * H * W, G = gridDim.x * RL;
-    for (int r = blockIdx.x * RL + rl; r < R; r += G) {
-        const int w = r % W, q = r / W, h = q % H, n = q / H;
-        float xv[8], g[8], o[8];
-        unpack8(ldg_nc_v4(x + (size_t)r * C + cg * 8), xv);
-        pooled_grad(dp, idx, n, h, w, cg, C, Ho, Wo, g);
-#pragma unroll
-        for (int k = 0; k < 8; ++k) {
-            const float gg = fmaf(xv[k], sc[k], bi[k]) > 0.f ? g[k] : 0.f;
-            o[k] = fmaf(c0[k], gg, fmaf(c1[k], xv[k], c2[k]));
-        }
-        store8(dx + (size_t)r * C + cg * 8, o);
-    }
-}
-
 static inline bool shape_ok(int C) {
     const int cg = C >> 3;
     return C % 8 == 0 && cg >= 1 && cg <= THREADS && (cg & (cg - 1)) == 0;     // 8, 16, ..., 2048
@@ -444,11 +279,11 @@ static inline bool shape_ok(int C) {
 // element-wise passes keep no partials: exactly one wave of resident CTAs (occupancy queried once per instantiation),
 // fewer when the tensor has fewer row groups than that
 template <typename K>
-static int apply_grid(K kernel, size_t smem, long long R, int C) {
+static int apply_grid(K kernel, long long R, int C) {
     int dev = 0, sms = 148, occ = 1;
     cudaGetDevice(&dev);
     cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
-    if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, kernel, THREADS, smem) != cudaSuccess || occ < 1) occ = 1;
+    if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, kernel, THREADS, 0) != cudaSuccess || occ < 1) occ = 1;
     const int RL = THREADS / (C >> 3);
     const long long g = (R + RL - 1) / RL, cap = (long long)occ * sms;
     return (int)(g < 1 ? 1 : (g > cap ? cap : g));
@@ -456,12 +291,11 @@ static int apply_grid(K kernel, size_t smem, long long R, int C) {
 
 // launch `kernel` as a programmatic dependent of the previous kernel in the stream (V6B200_PDL=0 or pdl=false: plain launch)
 template <typename... KArgs, typename... Args>
-static void launch_dependent(void (*kernel)(KArgs...), int grid, size_t smem, bool dependent, cudaStream_t s, Args... args) {
+static void launch_dependent(void (*kernel)(KArgs...), int grid, bool dependent, cudaStream_t s, Args... args) {
     static const bool pdl = [] { const char* e = getenv("V6B200_PDL"); return !(e && e[0] == '0'); }();
     cudaLaunchConfig_t cfg = {};
     cfg.gridDim = dim3((unsigned)grid);
     cfg.blockDim = dim3(THREADS);
-    cfg.dynamicSmemBytes = smem;
     cfg.stream = s;
     cudaLaunchAttribute attr[1];
     attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
@@ -471,7 +305,7 @@ static void launch_dependent(void (*kernel)(KArgs...), int grid, size_t smem, bo
     cudaLaunchKernelEx(&cfg, kernel, static_cast<KArgs>(args)...);
 }
 
-// same, 2-D grid, no dynamic shared memory (the reduce kernels)
+// same, 2-D grid (the reduce kernels)
 template <typename... KArgs, typename... Args>
 static void launch_dependent_grid(void (*kernel)(KArgs...), dim3 grid, cudaStream_t s, Args... args) {
     static const bool pdl = [] { const char* e = getenv("V6B200_PDL"); return !(e && e[0] == '0'); }();
@@ -487,47 +321,18 @@ static void launch_dependent_grid(void (*kernel)(KArgs...), dim3 grid, cudaStrea
     cudaLaunchKernelEx(&cfg, kernel, static_cast<KArgs>(args)...);
 }
 
-// tuning variant of the element-wise passes (V6B200_BN_CFG; scripts/bn_bench.py sweeps it, profiles/bn_bench_r2f.jsonl):
-//   0  U = 4 rows in flight, coefficients in shared memory, 4 CTAs/SM      2.93 ms of BN passes per ResNet-50 step
-//   1  U = 2, coefficients in registers, 3 CTAs/SM                          2.52 ms   (default; 5.5-6.0 TB/s on the
-//   2  U = 4, coefficients in registers, 2 CTAs/SM                          2.51 ms    100 MB layers = 0.84-0.91 of copy peak)
-static int bn_cfg() {
-    static const int v = [] { const char* e = getenv("V6B200_BN_CFG"); return e ? atoi(e) : 1; }();
-    return v;
-}
-
 template <bool RELU, bool RES>
 static void launch_apply(bool dependent, cudaStream_t s, const __nv_bfloat16* x, const __nv_bfloat16* res, const float* scale, const float* bias,
                          __nv_bfloat16* y, unsigned char* mask, long long R, int C) {
-    const int cfg = bn_cfg();
-    if (cfg == 1) {
-        auto k = bn_apply_kernel<RELU, RES, 2, 3, false>;
-        launch_dependent(k, apply_grid(k, 0, R, C), 0, dependent, s, x, res, scale, bias, y, mask, R, C);
-    } else if (cfg == 2) {
-        auto k = bn_apply_kernel<RELU, RES, 4, 2, false>;
-        launch_dependent(k, apply_grid(k, 0, R, C), 0, dependent, s, x, res, scale, bias, y, mask, R, C);
-    } else {
-        auto k = bn_apply_kernel<RELU, RES, 4, 4, true>;
-        const size_t sm = (size_t)2 * C * sizeof(float);
-        launch_dependent(k, apply_grid(k, sm, R, C), sm, dependent, s, x, res, scale, bias, y, mask, R, C);
-    }
+    auto k = bn_apply_kernel<RELU, RES, 2, 3>;
+    launch_dependent(k, apply_grid(k, R, C), dependent, s, x, res, scale, bias, y, mask, R, C);
 }
 
 template <bool RELU, bool RES>
 static void launch_bwd_apply(cudaStream_t s, const __nv_bfloat16* dy, const unsigned char* mask, const __nv_bfloat16* x, const float* coef,
                              __nv_bfloat16* dx, __nv_bfloat16* dres, long long R, int C) {
-    const int cfg = bn_cfg();
-    if (cfg == 1) {
-        auto k = bn_bwd_apply_kernel<RELU, RES, 2, 3, false>;
-        launch_dependent(k, apply_grid(k, 0, R, C), 0, true, s, dy, mask, x, coef, dx, dres, R, C);
-    } else if (cfg == 2) {
-        auto k = bn_bwd_apply_kernel<RELU, RES, 4, 2, false>;
-        launch_dependent(k, apply_grid(k, 0, R, C), 0, true, s, dy, mask, x, coef, dx, dres, R, C);
-    } else {
-        auto k = bn_bwd_apply_kernel<RELU, RES, 4, 4, true>;
-        const size_t sm = (size_t)3 * C * sizeof(float);
-        launch_dependent(k, apply_grid(k, sm, R, C), sm, true, s, dy, mask, x, coef, dx, dres, R, C);
-    }
+    auto k = bn_bwd_apply_kernel<RELU, RES, 2, 3>;
+    launch_dependent(k, apply_grid(k, R, C), true, s, dy, mask, x, coef, dx, dres, R, C);
 }
 
 }  // namespace bn
@@ -606,61 +411,6 @@ extern "C" int v6_bn_bwd(const void* dy, const void* relu_mask, const void* x, c
         if (dres) launch_bwd_apply<false, true>(s, dyy, yy, xx, coef, dxx, drr, R, C);
         else launch_bwd_apply<false, false>(s, dyy, yy, xx, coef, dxx, drr, R, C);
     }
-    V6_CHECK_LAUNCH();
-    return 0;
-}
-
-// element-wise half of the backward alone: the reduction (dgamma, dbeta, coef) was done in the epilogue of the data-gradient
-// kernel that produced dy (igemm.cu EPI_RED).  coef: [3C] = c0 | c1 | c2.
-extern "C" int v6_bn_bwd_apply(const void* dy, const void* relu_mask, const void* x, const float* coef, void* dx, void* dres, long long R,
-                               int C, int relu, cudaStream_t s) {
-    using namespace bn;
-    if (!shape_ok(C) || (relu && !relu_mask)) return (int)cudaErrorInvalidValue;
-    const __nv_bfloat16* dyy = (const __nv_bfloat16*)dy;
-    const unsigned char* yy = (const unsigned char*)relu_mask;
-    const __nv_bfloat16* xx = (const __nv_bfloat16*)x;
-    __nv_bfloat16* dxx = (__nv_bfloat16*)dx;
-    __nv_bfloat16* drr = (__nv_bfloat16*)dres;
-    if (relu) {
-        if (dres) launch_bwd_apply<true, true>(s, dyy, yy, xx, coef, dxx, drr, R, C);
-        else launch_bwd_apply<true, false>(s, dyy, yy, xx, coef, dxx, drr, R, C);
-    } else {
-        if (dres) launch_bwd_apply<false, true>(s, dyy, yy, xx, coef, dxx, drr, R, C);
-        else launch_bwd_apply<false, false>(s, dyy, yy, xx, coef, dxx, drr, R, C);
-    }
-    V6_CHECK_LAUNCH();
-    return 0;
-}
-
-// stem: y = maxpool3x3s2p1(relu(x * scale + bias)), idx = arg-max bytes.  x: [N, H, W, C] NHWC bf16, C % 64 == 0, C <= 2048 / CG <= 256.
-extern "C" int v6_bn_pool_fwd(const void* x, const float* scale, const float* bias, void* p, void* idx, int N, int H, int W, int C,
-                              cudaStream_t s) {
-    using namespace bn;
-    if (C % 64 != 0 || N < 1 || H < 2 || W < 2 || (long long)N * H * W * C >= (1LL << 31)) return (int)cudaErrorInvalidValue;
-    const int Ho = (H - 1) / 2 + 1, Wo = (W - 1) / 2 + 1;
-    const long long work = (long long)N * Ho * Wo * (C >> 3);
-    long long g = (work + THREADS - 1) / THREADS;
-    const int grid = (int)(g > 148 * 16 ? 148 * 16 : g);
-    launch_dependent(bn_relu_maxpool_fwd_kernel, grid, 0, true, s, (const __nv_bfloat16*)x, scale, bias, (__nv_bfloat16*)p, (unsigned char*)idx,
-                     N, H, W, C, Ho, Wo);
-    V6_CHECK_LAUNCH();
-    return 0;
-}
-
-extern "C" int v6_bn_pool_bwd(const void* dp, const void* idx, const void* x, const float* scale, const float* bias, const float* gamma,
-                              const float* mean, const float* rstd, void* dx, float* dgamma, float* dbeta, float* coef, float* scratch,
-                              int N, int H, int W, int C, int accumulate, cudaStream_t s) {
-    using namespace bn;
-    if (C % 64 != 0 || !shape_ok(C) || (long long)N * H * W * C >= (1LL << 31)) return (int)cudaErrorInvalidValue;
-    const int Ho = (H - 1) / 2 + 1, Wo = (W - 1) / 2 + 1;
-    const long long R = (long long)N * H * W;
-    static int wave = 0;
-    const dim3 rg = reduce_grid(R, C, wave_ctas(bn_pool_bwd_reduce_kernel, wave));
-    launch_dependent_grid(bn_pool_bwd_reduce_kernel, rg, s, (const __nv_bfloat16*)dp, (const unsigned char*)idx, (const __nv_bfloat16*)x, scale, bias,
-                          gamma, mean, rstd, make_red(scratch), dgamma, dbeta, coef, N, H, W, C, Ho, Wo, accumulate);
-    auto k = bn_pool_bwd_apply_kernel;
-    launch_dependent(k, apply_grid(k, 0, R, C), 0, true, s, (const __nv_bfloat16*)dp, (const unsigned char*)idx, (const __nv_bfloat16*)x, scale, bias,
-                     (const float*)coef, (__nv_bfloat16*)dx, N, H, W, C, Ho, Wo);
     V6_CHECK_LAUNCH();
     return 0;
 }

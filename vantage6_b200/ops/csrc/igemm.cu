@@ -101,12 +101,6 @@ struct Params {
     float* mean_out; float* rstd_out; float* scale_out; float* bias_out;
     float* part; int* counters; float eps, momentum;
     int stat_arrivals;       // CTAs that publish sums for one column block
-    // DGRAD + BatchNorm backward reduction (EPI_RED): the BN whose output gradient this kernel produces
-    const __nv_bfloat16* red_x;        // [M, N] its input (the convolution output it normalised)
-    const unsigned char* red_mask;     // [M, N/8] ReLU mask of its output (null: no ReLU)
-    const float* red_mean; const float* red_rstd; const float* red_gamma;
-    float* red_dgamma; float* red_dbeta; float* red_coef;      // coef: [3N] = c0 | c1 | c2 of dx = c0 g + c1 x + c2
-    int red_accumulate;                // dgamma / dbeta += (flat gradient buffer) instead of =
 };
 
 V6_DEVINL float gelu_erf(float x) { return 0.5f * x * (1.f + erff(x * 0.70710678118654752f)); }
@@ -196,10 +190,7 @@ struct Item { int m_blk, n_blk, kb0, kb1, cls; };
 //   EPI_PLAIN  bf16 tile -> staging -> TMA store
 //   EPI_STATS  + BatchNorm statistics of the tile (FPROP)
 //   EPI_GEN    bias / activation / add_src / stride-2 scatter
-//   EPI_RED    DGRAD (stride 1, optional add_src): + the reduction pass of the BatchNorm backward that consumes this
-//              gradient -- sum g and sum g.xhat per channel with g = dx . relu'(y), finalised to dgamma / dbeta and the
-//              coefficients of the BN data gradient (bn.cu::bn_bwd_reduce_kernel disappears for that layer)
-enum { EPI_PLAIN = 0, EPI_STATS = 1, EPI_GEN = 2, EPI_RED = 3 };
+enum { EPI_PLAIN = 0, EPI_STATS = 1, EPI_GEN = 2 };
 
 template <int MODE, int EPI>
 __global__ void __launch_bounds__(kThreads, 1)
@@ -233,7 +224,7 @@ igemm_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_constant__
         Item it;
         it.cls = 0;
         const int tile = (MODE == WGRAD || strided) ? item % num_tiles : item;
-        if (EPI == EPI_STATS || EPI == EPI_RED) {
+        if (EPI == EPI_STATS) {
             // n fastest and gridDim.x a multiple of num_n (host): a CTA stays on ONE column block for all of its row tiles, so
             // its per-channel running sums leave the registers once, at the end
             it.n_blk = tile % num_n;
@@ -405,12 +396,6 @@ igemm_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_constant__
         const int half = warp >> 2;             // this warp takes the 32-column chunks with (chunk & 1) == half
         const int et = warp * 32 + lane;        // epilogue thread id 0..255: owns column `et` of the statistics
         constexpr bool stats = MODE == FPROP && EPI == EPI_STATS;
-        constexpr bool red = MODE == DGRAD && EPI == EPI_RED;
-        // EPI_RED: per-lane sums over the rows this lane stores (rows lane>>2 + 8i of every box), of its 8 channels
-        // (lane & 3) of chunk slot 0 (ra) / 1 (rb): block_n <= 128 for this epilogue (host), so two slots cover a tile
-        float ra1[8], ra2[8], rb1[8], rb2[8];
-#pragma unroll
-        for (int e = 0; e < 8; ++e) ra1[e] = ra2[e] = rb1[e] = rb2[e] = 0.f;
         int acc = 0; uint32_t acc_phase = 0;
         float run1[4][2], run2[4][2];                 // running column sums of this warp's (<= 4) chunks: lanes 0..15 own a column pair
 #pragma unroll
@@ -452,12 +437,12 @@ igemm_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_constant__
         // staging box -> global memory: 4 lanes cover one row's 64 bytes (two full 32-byte sectors), 8 rows per instruction.
         // (v2 used a TMA store per box: its proxy fence + store-read wait sat on the critical path of every chunk and the
         // short-K layers are bound by exactly this chain -- profiles/ncu_igemm_r2b.md.)
-        auto box_to_global = [&](uint32_t sbox, int row0, int c0, float (&r1)[8], float (&r2)[8]) {
+        auto box_to_global = [&](uint32_t sbox, int row0, int c0) {
             const int ch = lane & 3;
             if (c0 + ch * 8 >= P.N) return;
             const size_t off = (size_t)(row0 + (lane >> 2)) * P.N + c0 + ch * 8;
             uint4 val[4], addv[4];
-            const bool add = (EPI == EPI_GEN || EPI == EPI_RED) && P.add_src != nullptr;
+            const bool add = EPI == EPI_GEN && P.add_src != nullptr;
             unsigned mbits[4] = {0xffu, 0xffu, 0xffu, 0xffu};
             if (add) {      // the gradient of the residual branch, read with the same fully coalesced pattern as the store
 #pragma unroll
@@ -489,38 +474,6 @@ igemm_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_constant__
 #pragma unroll
             for (int i = 0; i < 4; ++i)
                 if (row0 + (lane >> 2) + 8 * i < P.M) *reinterpret_cast<uint4*>(dst + (size_t)(8 * i) * P.N) = val[i];
-            if (red) {
-                // BatchNorm backward reduction on the gradient just stored: g = dx where the ReLU mask of the BN output is set;
-                // x = the BN input, read with the same coalesced pattern.  sum g -> r1, sum g (x - mean) rstd -> r2
-                float mu[8], rsd[8];
-                {
-                    const float4 m0 = __ldg(reinterpret_cast<const float4*>(P.red_mean + c0 + ch * 8)), m1 = __ldg(reinterpret_cast<const float4*>(P.red_mean + c0 + ch * 8 + 4));
-                    const float4 s0 = __ldg(reinterpret_cast<const float4*>(P.red_rstd + c0 + ch * 8)), s1 = __ldg(reinterpret_cast<const float4*>(P.red_rstd + c0 + ch * 8 + 4));
-                    mu[0] = m0.x; mu[1] = m0.y; mu[2] = m0.z; mu[3] = m0.w; mu[4] = m1.x; mu[5] = m1.y; mu[6] = m1.z; mu[7] = m1.w;
-                    rsd[0] = s0.x; rsd[1] = s0.y; rsd[2] = s0.z; rsd[3] = s0.w; rsd[4] = s1.x; rsd[5] = s1.y; rsd[6] = s1.z; rsd[7] = s1.w;
-                }
-                uint4 xr[4];
-                unsigned mb[4];
-#pragma unroll
-                for (int i = 0; i < 4; ++i) {
-                    const bool in = row0 + (lane >> 2) + 8 * i < P.M;
-                    xr[i] = in ? __ldg(reinterpret_cast<const uint4*>(P.red_x + off + (size_t)(8 * i) * P.N)) : make_uint4(0u, 0u, 0u, 0u);
-                    mb[i] = !in ? 0u : (P.red_mask ? (unsigned)__ldg(P.red_mask + (off + (size_t)(8 * i) * P.N) / 8) : 0xffu);
-                }
-#pragma unroll
-                for (int i = 0; i < 4; ++i) {
-                    const uint32_t* gv = reinterpret_cast<const uint32_t*>(&val[i]);
-                    const uint32_t* xv = reinterpret_cast<const uint32_t*>(&xr[i]);
-#pragma unroll
-                    for (int e = 0; e < 4; ++e) {
-                        const float2 g = unpack_bf16x2(gv[e]), x = unpack_bf16x2(xv[e]);
-                        const float g0 = ((mb[i] >> (2 * e)) & 1u) ? g.x : 0.f, g1 = ((mb[i] >> (2 * e + 1)) & 1u) ? g.y : 0.f;
-                        r1[2 * e] += g0; r1[2 * e + 1] += g1;
-                        r2[2 * e] = fmaf(g0, (x.x - mu[2 * e]) * rsd[2 * e], r2[2 * e]);
-                        r2[2 * e + 1] = fmaf(g1, (x.y - mu[2 * e + 1]) * rsd[2 * e + 1], r2[2 * e + 1]);
-                    }
-                }
-            }
         };
         // column sums of the bf16-rounded box: lanes 0..15 take rows 0..15, lanes 16..31 rows 16..31 of column pair
         // (lane & 15); the halves meet through one shuffle; added to the running sums of chunk slot k
@@ -633,8 +586,8 @@ igemm_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_constant__
                         if (second) box_scatter(stg + STG_BOX_BYTES, row0, c1, it.cls);
                         continue;
                     }
-                    box_to_global(stg, row0, c0, ra1, ra2);
-                    if (second) box_to_global(stg + STG_BOX_BYTES, row0, c1, rb1, rb2);
+                    box_to_global(stg, row0, c0);
+                    if (second) box_to_global(stg + STG_BOX_BYTES, row0, c1);
                     if (stats) { box_stats(stg, k); if (second) box_stats(stg + STG_BOX_BYTES, k + 1); }
                 }
                 if (k < nck) {                                               // odd chunk count (block_n = 64 / 192)
@@ -651,7 +604,7 @@ igemm_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_constant__
                         if (EPI == EPI_GEN && strided) {
                             box_scatter(stg, row0, c0, it.cls);
                         } else {
-                            box_to_global(stg, row0, c0, ra1, ra2);
+                            box_to_global(stg, row0, c0);
                             if (stats) box_stats(stg, k);
                         }
                     }
@@ -662,7 +615,7 @@ igemm_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_constant__
             if (lane == 0) mbar_arrive(&tempty_bar[acc]);
             if (++acc == kAccStages) { acc = 0; acc_phase ^= 1; }
 
-            if (stats || red) {
+            if (stats) {
                 const int nxt = item + gridDim.x;
                 const bool flush = nxt >= num_items || decode(nxt).n_blk != it.n_blk;
                 if (flush) {
@@ -670,38 +623,15 @@ igemm_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_constant__
                     // column block's; the last CTA to arrive finalizes
                     __syncwarp();
                     // this warp's box area doubles as scratch: [chunk k][sum | sumsq][32 columns] floats = 1 KB of the 4 KB
-                    if (stats) {
-                        if (lane < 16) {
+                    if (lane < 16) {
 #pragma unroll
-                            for (int k = 0; k < 4; ++k) {
-                                sts_f2(stg + (k * 64 + 2 * lane) * 4, run1[k][0], run1[k][1]);
-                                sts_f2(stg + (k * 64 + 32 + 2 * lane) * 4, run2[k][0], run2[k][1]);
-                            }
+                        for (int k = 0; k < 4; ++k) {
+                            sts_f2(stg + (k * 64 + 2 * lane) * 4, run1[k][0], run1[k][1]);
+                            sts_f2(stg + (k * 64 + 32 + 2 * lane) * 4, run2[k][0], run2[k][1]);
                         }
-#pragma unroll
-                        for (int k = 0; k < 4; ++k) run1[k][0] = run1[k][1] = run2[k][0] = run2[k][1] = 0.f;
-                    } else {
-                        // the 8 lanes that share a channel group (same lane & 3, different rows) meet by shuffles; lanes 0-3 write
-#pragma unroll
-                        for (int e = 0; e < 8; ++e) {
-#pragma unroll
-                            for (int sh = 4; sh < 32; sh <<= 1) {
-                                ra1[e] += __shfl_xor_sync(0xffffffffu, ra1[e], sh); ra2[e] += __shfl_xor_sync(0xffffffffu, ra2[e], sh);
-                                rb1[e] += __shfl_xor_sync(0xffffffffu, rb1[e], sh); rb2[e] += __shfl_xor_sync(0xffffffffu, rb2[e], sh);
-                            }
-                        }
-                        if (lane < 4) {
-#pragma unroll
-                            for (int e = 0; e < 8; e += 2) {
-                                sts_f2(stg + (0 * 64 + lane * 8 + e) * 4, ra1[e], ra1[e + 1]);
-                                sts_f2(stg + (0 * 64 + 32 + lane * 8 + e) * 4, ra2[e], ra2[e + 1]);
-                                sts_f2(stg + (1 * 64 + lane * 8 + e) * 4, rb1[e], rb1[e + 1]);
-                                sts_f2(stg + (1 * 64 + 32 + lane * 8 + e) * 4, rb2[e], rb2[e + 1]);
-                            }
-                        }
-#pragma unroll
-                        for (int e = 0; e < 8; ++e) ra1[e] = ra2[e] = rb1[e] = rb2[e] = 0.f;
                     }
+#pragma unroll
+                    for (int k = 0; k < 4; ++k) run1[k][0] = run1[k][1] = run2[k][0] = run2[k][1] = 0.f;
                     epi_bar_sync();
                     double* sums = reinterpret_cast<double*>(P.part) + (size_t)it.n_blk * P.block_n * 2;
                     if (et < P.block_n) {
@@ -734,20 +664,7 @@ igemm_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_constant__
                         __stcg(sums + et, 0.0);                          // self-resetting, like the counters
                         __stcg(sums + P.block_n + et, 0.0);
                         const int c = it.n_blk * P.block_n + et;
-                        if (red) {
-                            if (c < P.N) {
-                                // t1 = sum g, t2 = sum g.xhat (bn.cu::bn_bwd_reduce_kernel's finalize)
-                                const float tg = (float)t1, tgx = (float)t2;
-                                P.red_dgamma[c] = P.red_accumulate ? P.red_dgamma[c] + tgx : tgx;
-                                P.red_dbeta[c] = P.red_accumulate ? P.red_dbeta[c] + tg : tg;
-                                const float invR = 1.f / (float)P.M, rs_c = P.red_rstd[c];
-                                const float k0 = P.red_gamma[c] * rs_c;
-                                const float k1 = -k0 * rs_c * tgx * invR;
-                                P.red_coef[c] = k0;
-                                P.red_coef[P.N + c] = k1;
-                                P.red_coef[2 * P.N + c] = -k0 * tg * invR - k1 * P.red_mean[c];
-                            }
-                        } else if (c < P.N) {
+                        if (c < P.N) {
                             const double invR = 1.0 / (double)P.M;
                             const double mean_d = t1 * invR;
                             double var_d = t2 * invR - mean_d * mean_d;
@@ -797,7 +714,7 @@ typedef void (*KernelFn)(const CUtensorMap, const CUtensorMap, const CUtensorMap
 KernelFn pick_kernel(int mode, int epi) {
     using namespace igemm;
     if (mode == FPROP) return epi == EPI_STATS ? igemm_kernel<FPROP, EPI_STATS> : epi == EPI_GEN ? igemm_kernel<FPROP, EPI_GEN> : igemm_kernel<FPROP, EPI_PLAIN>;
-    if (mode == DGRAD) return epi == EPI_GEN ? igemm_kernel<DGRAD, EPI_GEN> : epi == EPI_RED ? igemm_kernel<DGRAD, EPI_RED> : igemm_kernel<DGRAD, EPI_PLAIN>;
+    if (mode == DGRAD) return epi == EPI_GEN ? igemm_kernel<DGRAD, EPI_GEN> : igemm_kernel<DGRAD, EPI_PLAIN>;
     return igemm_kernel<WGRAD, EPI_PLAIN>;
 }
 
@@ -805,8 +722,7 @@ int set_smem_attr() {
     static bool done = false;
     if (!done) {
         using namespace igemm;
-        const int combos[7][2] = {{FPROP, EPI_PLAIN}, {FPROP, EPI_STATS}, {FPROP, EPI_GEN}, {DGRAD, EPI_PLAIN}, {DGRAD, EPI_GEN}, {DGRAD, EPI_RED},
-                                  {WGRAD, EPI_PLAIN}};
+        const int combos[6][2] = {{FPROP, EPI_PLAIN}, {FPROP, EPI_STATS}, {FPROP, EPI_GEN}, {DGRAD, EPI_PLAIN}, {DGRAD, EPI_GEN}, {WGRAD, EPI_PLAIN}};
         for (auto& c : combos) {
             cudaError_t e = cudaFuncSetAttribute(pick_kernel(c[0], c[1]), cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_BYTES);
             if (e != cudaSuccess) return (int)e;
@@ -854,9 +770,9 @@ int launch(int mode, const CUtensorMap& ta, const CUtensorMap& tb, const CUtenso
     int grid = items < cap ? items : cap;
     int epi = EPI_PLAIN;
     if (mode == FPROP) epi = P.gamma ? EPI_STATS : ((P.bias || P.act) ? EPI_GEN : EPI_PLAIN);
-    else if (mode == DGRAD) epi = P.red_x ? EPI_RED : ((P.dstride == 2 || P.add_src) ? EPI_GEN : EPI_PLAIN);
+    else if (mode == DGRAD) epi = (P.dstride == 2 || P.add_src) ? EPI_GEN : EPI_PLAIN;
     igemm::Params Pl = P;
-    if (epi == EPI_STATS || epi == EPI_RED) {      // every CTA keeps one column block (see decode): grid = whole groups of num_n CTAs
+    if (epi == EPI_STATS) {      // every CTA keeps one column block (see decode): grid = whole groups of num_n CTAs
         grid = items < cap ? items : (cap / num_n) * num_n;
         Pl.stat_arrivals = grid / num_n;
     }
@@ -915,12 +831,9 @@ extern "C" int v6_conv_fprop(const void* x, const void* w, void* y, const float*
 
 // dx[N,H,W,Cin] = conv_transpose(dy[N,P,Q,Cout], w[Cout,R,S,Cin]) for stride 1 (P = H + 2*pad - R + 1)
 extern "C" int v6_conv_dgrad(const void* dy, const void* w, void* dx, int N, int H, int W, int Cin, int Cout, int R, int S, int stride,
-                             int pad, int force_im2col, const void* add_src, const void* add_mask, const void* red_x, const void* red_mask,
-                             const float* red_mean, const float* red_rstd, const float* red_gamma, float* red_dgamma, float* red_dbeta,
-                             float* red_coef, int red_accumulate, float* scratch, cudaStream_t stream) {
+                             int pad, int force_im2col, const void* add_src, const void* add_mask, cudaStream_t stream) {
     using namespace igemm;
     if (Cout % 64 != 0 || Cin % 8 != 0 || R != S) return (int)cudaErrorInvalidValue;
-    if (red_x && (stride != 1 || Cin % 64 != 0 || !scratch || Cin > 2048)) return (int)cudaErrorInvalidValue;
     if (add_src && (stride != 1 || Cin % 32 != 0)) return (int)cudaErrorInvalidValue;
     alignas(64) CUtensorMap ta, tb, tc;
     {
@@ -975,12 +888,6 @@ extern "C" int v6_conv_dgrad(const void* dy, const void* w, void* dx, int N, int
     P.M = M; P.N = Cin; P.num_kb = R * S * (Cout / 64); P.block_n = pick_block_n(M, Cin, R * S * (Cout / 64));
     P.a_im2col = plain ? 0 : 1; P.PQ = H * W; P.Q = W; P.stride = 1; P.pad = R - 1 - pad; P.S = S; P.cblocks = Cout / 64; P.taps = R * S; P.flip = 1;
     P.dstride = 1; P.add_src = (const __nv_bfloat16*)add_src; P.add_mask = add_src ? (const unsigned char*)add_mask : nullptr; P.c_out = (__nv_bfloat16*)dx;
-    if (red_x) {       // + the reduction pass of the BatchNorm backward that consumes dx (EPI_RED; two chunk slots per warp: block_n <= 128)
-        if (P.block_n > 128) P.block_n = 128;
-        P.red_x = (const __nv_bfloat16*)red_x; P.red_mask = (const unsigned char*)red_mask; P.red_mean = red_mean; P.red_rstd = red_rstd;
-        P.red_gamma = red_gamma; P.red_dgamma = red_dgamma; P.red_dbeta = red_dbeta; P.red_coef = red_coef; P.red_accumulate = red_accumulate;
-        P.counters = reinterpret_cast<int*>(scratch); P.part = scratch + 64;
-    }
     if (plain) { if (v6_make_tmap_2d_bf16(&ta, (uint64_t)dy, M, Cout, (uint64_t)Cout * 2, BLOCK_M, BLOCK_K, 1)) return -2; }
     else { ConvGeom g{N, Pp, Qq, Cout, R, S, 1, R - 1 - pad, H, W}; if (im2col_map(&ta, dy, g, BLOCK_M)) return -2; }
     if (v6_make_tmap_2d_bf16(&tc, (uint64_t)dx, M, Cin, (uint64_t)Cin * 2, 32, 32, 2)) return -2;

@@ -227,18 +227,6 @@ PYBIND11_MODULE(_C, m) {
     m.def("ce_bwd", [](u64 logits, u64 labels, u64 lse, u64 scale, int T, int V, int V_alloc, long long ld, long long ignore_index, u64 s) {
         check(v6_ce_bwd(P<void>(logits), P<long long>(labels), P<float>(lse), P<float>(scale), T, V, V_alloc, ld, ignore_index, S(s)), "ce_bwd");
     });
-    m.def("bn_pool_fwd", [](u64 x, u64 scale, u64 bias, u64 p, u64 idx, int N, int H, int W, int C, u64 s) {
-        check(v6_bn_pool_fwd(P<void>(x), P<float>(scale), P<float>(bias), P<void>(p), P<void>(idx), N, H, W, C, S(s)), "bn_pool_fwd");
-    });
-    m.def("bn_pool_bwd", [](u64 dp, u64 idx, u64 x, u64 scale, u64 bias, u64 gamma, u64 mean, u64 rstd, u64 dx, u64 dgamma, u64 dbeta, u64 coef,
-                            u64 scratch, int N, int H, int W, int C, bool accumulate, u64 s) {
-        check(v6_bn_pool_bwd(P<void>(dp), P<void>(idx), P<void>(x), P<float>(scale), P<float>(bias), P<float>(gamma), P<float>(mean), P<float>(rstd),
-                             P<void>(dx), P<float>(dgamma), P<float>(dbeta), P<float>(coef), P<float>(scratch), N, H, W, C, accumulate ? 1 : 0, S(s)),
-              "bn_pool_bwd");
-    });
-    m.def("bn_bwd_apply", [](u64 dy, u64 mask, u64 x, u64 coef, u64 dx, u64 dres, long long R, int C, bool relu, u64 s) {
-        check(v6_bn_bwd_apply(P<void>(dy), P<void>(mask), P<void>(x), P<float>(coef), P<void>(dx), P<void>(dres), R, C, relu, S(s)), "bn_bwd_apply");
-    });
     m.attr("BN_SCRATCH_FLOATS") = v6_bn_scratch_floats();
 
     // ------------------------------------------------------------------ K6 / K8
@@ -276,11 +264,9 @@ PYBIND11_MODULE(_C, m) {
               "conv_fprop");
     });
     m.def("conv_dgrad", [](u64 dy, u64 w, u64 dx, int N, int H, int W, int Cin, int Cout, int R, int Sw, int stride, int pad,
-                           bool force_im2col, u64 s, u64 add_src, u64 add_mask, u64 red_x, u64 red_mask, u64 red_mean, u64 red_rstd,
-                           u64 red_gamma, u64 red_dgamma, u64 red_dbeta, u64 red_coef, bool red_accumulate, u64 scratch) {
+                           bool force_im2col, u64 s, u64 add_src, u64 add_mask) {
         check(v6_conv_dgrad(P<void>(dy), P<void>(w), P<void>(dx), N, H, W, Cin, Cout, R, Sw, stride, pad, force_im2col, P<void>(add_src), P<void>(add_mask),
-                            P<void>(red_x), P<void>(red_mask), P<float>(red_mean), P<float>(red_rstd), P<float>(red_gamma), P<float>(red_dgamma),
-                            P<float>(red_dbeta), P<float>(red_coef), red_accumulate ? 1 : 0, P<float>(scratch), S(s)), "conv_dgrad");
+                            S(s)), "conv_dgrad");
     });
     m.def("conv_wgrad", [](u64 dy, u64 x, u64 dw, int N, int H, int W, int Cin, int Cout, int R, int Sw, int stride, int pad,
                            float scale, int splits, bool force_im2col, u64 s, long long pitch_w, long long pitch_h, long long pitch_n,
